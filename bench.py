@@ -6,8 +6,9 @@ fine-stage HBM roofline, next to the CPU baseline (the oracle = restated referen
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W          (one rank per GPU, tile-row stripes assembled over NVLink)
     python bench.py --impl reference ...                (the CPU arm: oracle on the host cores)
+    python bench.py ... --dump-outputs DIR              (also write the last timed frame to DIR, see dump_outputs)
 
-One step = one frame of the hot path (pathtag .. fine) over the synthetic scene.
+One step = one frame of the hot path (pathtag .. fine) over the synthetic scene; --steps is the number of timed steps.
 `value`  : frames/s with the packed scene already resident in HBM (vb_render_resident).
 `e2e`    : frames/s through the C ABI with pinned HOST buffers (streaming `vb_render_begin`; the blocking one-call
            `vb_render` figure is reported next to it): scene H2D + render +
@@ -54,6 +55,21 @@ def build_scene(args):
         sc = scenes.paris_like(args.paths, args.size, args.seed)
     packed = resolve(sc.encoding)
     return packed, time.time() - t
+
+
+DUMP_BYTES = 48 << 20  # float32 pixels per dump: with the row indices, a dump stays below 64 MB
+
+
+def dump_outputs(out_dir, frame):
+    """Write the frame of the last timed step (RGBA8, un-premultiplied) as float32 `frame.npy`, shape (rows, width, 4), and
+    the frame rows it holds as float64 `frame_rows.npy`. A frame larger than DUMP_BYTES is sampled by rows chosen with a
+    fixed seed, so two builds run with the same arguments can be compared pixel for pixel."""
+    os.makedirs(out_dir, exist_ok=True)
+    h, w = frame.shape[:2]
+    n = max(1, min(h, DUMP_BYTES // (w * 4 * 4)))
+    rows = np.arange(h) if n == h else np.sort(np.random.default_rng(0).choice(h, n, replace=False))
+    np.save(os.path.join(out_dir, "frame.npy"), frame[rows].astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_rows.npy"), rows.astype(np.float64))
 
 
 class ClockSampler:
@@ -126,9 +142,9 @@ def run_cpu_arm(args, packed, as_reference):
     from vello_b200.encoding import BLACK
     cores = os.cpu_count() or 1
     o = Oracle(threads=cores)
-    # bounded sample: one full frame is ~3-5 s of CPU work on 8 cores, so the reference arm runs at most
-    # one warm-up frame and stops after ~2 minutes of timed frames
-    steps = max(1, min(args.steps, 20) if as_reference else 1)
+    # one full frame is ~3-5 s of CPU work on 8 cores, so the reference arm runs at most one warm-up frame; it times
+    # exactly --steps frames (the cpu_baseline beside the GPU figure times one)
+    steps = args.steps if as_reference else 1
     warm = min(args.warmup, 1) if as_reference else 0
     times, serial, fine = [], [], []
     w, h = args.size, args.height or args.size
@@ -144,8 +160,6 @@ def run_cpu_arm(args, packed, as_reference):
             times.append(t2 - t)
             serial.append(t1 - t)
             fine.append(t2 - t1)
-        if sum(times) > 120:
-            break
     fps = len(times) / sum(times)
     fine_threads = min(cores, 1024, (h + 15) // 16)
     return fps, dict(value=fps, unit="frames/s", cores=cores, kind="port",
@@ -188,7 +202,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-exchange", action="store_true", help="N > 1: every rank flattens the whole scene (round-1 behaviour)")
     ap.add_argument("--profile-only", action="store_true", help="just run warmup+steps resident frames (for ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if not args.profile_only else args.warmup
 
     H = args.height or args.size
@@ -202,7 +219,9 @@ def main():
         if rank != 0:
             return
         packed, _ = build_scene(args)
-        fps, cb, ms, n, _ = run_cpu_arm(args, packed, True)
+        fps, cb, ms, n, frame = run_cpu_arm(args, packed, True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, frame)
         emit({"impl": "reference", "metric": "frames/sec paris-30k@4K", "value": fps, "unit": "frames/s",
                           "n_gpus": args.gpus, "steps": n, "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True,
                           "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config,
@@ -265,6 +284,8 @@ def main():
     else:
         p2p_frame = True
     frame_base = int(frame_ptr.value or 0)
+    if args.dump_outputs and not p2p_frame:
+        raise SystemExit("--dump-outputs: the stripes stay on their GPUs (no peer mapping of rank 0's frame), so no rank holds the frame")
 
     bounds = even_tile_bounds(world, H)
 
@@ -445,6 +466,11 @@ def main():
     barrier()
     wall = time.perf_counter() - t_wall
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # read back now: the sections below render into the same frame
+        last = np.zeros((H, args.size, 4), dtype=np.uint8)
+        assert r.lib.vb_copy_to_host(r.handle, vp(frame_base), vp(last.ctypes.data), C.c_size_t(last.nbytes)) == 0
+        dump_outputs(args.dump_outputs, last)
+        del last
     step_ms = torch.tensor([a.elapsed_time(b) for a, b in evs], dtype=torch.float64, device=dev)
     my_total = float(step_ms.sum().item())
     if dist is not None:

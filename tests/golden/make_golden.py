@@ -1,4 +1,4 @@
-"""Generate the committed golden fixtures from the reference checkout (run HERE, not on the GPU box).
+"""Generate the committed golden fixtures from a checkout of the reference project (needs no GPU).
 
 * smoke_*.npy : the reference's in-repo snapshot PNGs (vello_tests/snapshots/smoke/*.png; the
   other snapshot directories are git-LFS pointers) decoded to RGBA8 arrays. They pin the oracle
@@ -9,7 +9,7 @@
   (examples/scenes/src/pico_svg.rs:134-195): per <path> the fill / stroke colours, stroke width
   and the path data string. The SVG itself is not copied.
 
-Usage: python tests/golden/make_golden.py [/root/reference]
+Usage: python tests/golden/make_golden.py <reference checkout>
 """
 import gzip
 import json
@@ -24,7 +24,7 @@ from PIL import Image
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def main(ref="/root/reference"):
+def main(ref):
     smoke = os.path.join(ref, "vello_tests/snapshots/smoke")
     for name in ["filled_square", "filled_circle", "layer_size", "gradient_color_alpha_premultiplied",
                  "gradient_color_alpha_unpremultiplied", "data_image_roundtrip"]:
@@ -62,4 +62,6 @@ def main(ref="/root/reference"):
 
 
 if __name__ == "__main__":
-    main(*sys.argv[1:])
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])
