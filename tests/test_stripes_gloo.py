@@ -74,7 +74,7 @@ def test_stripes_over_gloo(tmp_path, world):
 
 
 def test_tile_row_bounds_and_rebalance():
-    """The cost-balanced tile-row split (vello_b200.stripes.rebalance == group_rebalance in vb_api.cu): boundaries stay
+    """The cost-balanced tile-row split (vello_b200.stripes.rebalance == group_rebalance in vb_group.cu): boundaries stay
     monotone with at least one row per stripe, move towards the slower stripes, stop inside the tolerance, and converge on a
     synthetic cost profile."""
     from vello_b200.stripes import even_tile_bounds, n_tile_rows, rebalance

@@ -10,14 +10,11 @@
 #include <stdlib.h>
 #include <string.h>
 
-#include <algorithm>
 #include <string>
-#include <utility>
 #include <vector>
 
-#include "../../include/vello_b200.h"
 #include "vb_device.cuh"
-#include "vb_types.h"
+#include "vb_internal.h"
 
 // ---- stage launchers (k_*.cu) --------------------------------------------------------------
 extern "C" {
@@ -124,159 +121,40 @@ __global__ void k_publish_bump(const VbBump *bump, VbBump *host) {
     }
 }
 
-struct DevBuf {
-    void *p = nullptr;
-    size_t cap = 0; // bytes
-};
-
-// key of a captured frame: everything a launch argument is derived from (see enqueue)
-struct GraphKey {
-    VbConfig cfg;
-    const void *ptrs[32];
-    uint64_t ctl_words;
-    uint32_t aa, cull, last;
-    uint32_t xen, xrows[9];
-    const void *xpeer[8];
-};
-struct GraphSlot {
-    GraphKey key;
-    cudaGraphExec_t exec = nullptr;
-    uint32_t launches = 0;
-};
-
-struct vb_renderer {
-    int device = 0;
-    cudaStream_t stream = nullptr;
-    bool timing = false;
-    uint32_t max_retries = 6;
-    std::string err;
-    int sm_count = 148;
-
-    // scene
-    bool have_scene = false;
-    VbLayout layout{};
-    size_t scene_words = 0;
-    uint32_t n_ramps = 0, atlas_w = 0, atlas_h = 0;
-    DevBuf scene, ramps, atlas, mask8, mask16;
-
-    // fixed-size intermediates
-    DevBuf tag_monoids, path_bboxes, draw_monoids, info_bin_data, clip_inp, clip_bboxes, clip_scratch, draw_bboxes, bin_headers, paths,
-        ctl, target, target_alt, tile_start, cls_list;
-    // bump arenas (capacities in elements live in cap_*)
-    DevBuf resolve_tmp; // patches, ramp descriptors and stops of vb_scene_upload_streams
-    DevBuf lines, line_scratch, flatten_jobs, flatten_parts, tiles, seg_counts, segments, ptcl, blend_spill;
-    uint32_t cap_lines = 0, cap_binning = 0, cap_tiles = 0, cap_seg_counts = 0, cap_segments = 0, cap_blend = 0, cap_ptcl = 0;
-
-    // per-frame
-    VbConfig cfg{};
-    vb_params params{};
-    void *out_dev = nullptr;
-    VbBump *h_bump = nullptr;   // pinned + mapped: the device writes the counters straight into host memory
-    VbBump *h_bump_dev = nullptr; // device-side address of h_bump
-    uint32_t retries = 0, launches = 0;
-    size_t ctl_words = 0;
-    bool use_graph = true;        // replay whole frames as CUDA graphs (see enqueue)
-    GraphSlot graphs[4];
-    uint32_t graph_next = 0;
-    uint32_t readback_bands = 8; // fine launches per frame when the pixels go to the host (vb_render); 1 while streaming
-    uint32_t occlusion_cull = 1; // fine starts each tile at its last opaque full-tile cover
-    uint32_t parts_pathtag = 0, parts_flatten = 0, parts_draw = 0, parts_tile = 0;
-    size_t off_lb_pathtag = 0, off_lb_flatten = 0, off_lb_draw = 0, off_lb_tile = 0, off_lb_clip = 0;
-    cudaEvent_t ev[VB_N_STAGE_IDS + 1]{};
-    cudaEvent_t frame_ev[2]{}; // around every whole frame (vb_last_frame_ms: the signal stripe balancing uses)
-    bool frame_timed = false;
-    bool ev_ok = false;
-    // read-back pipeline of vb_render (host output): fine runs in row bands, each band's D2H copy overlaps the next band
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t band_ev[8]{};
-    void *host_out = nullptr; // set by vb_render for the duration of one frame
-    // streaming read-back (vb_render_begin): frames alternate between two targets so that the copy of frame n can
-    // still be draining while frame n+1 is rasterised
-    bool use_alt = false, stream_pending = false;
-    uint32_t stream_parity = 0;
-    cudaEvent_t copy_done[3]{};
-    bool frame_pending = false;
-    bool zero_fine_queue = false; // set by vb_run_stages (see enqueue_direct)
-    bool in_stream_call = false;  // inside vb_render_begin / vb_readback_wait (their internal calls must not drain)
-
-    // Streaming (vb_render_begin) keeps TWO frames in flight: while frame k is rasterised, frame k+1's scene is uploaded
-    // into the other slot on its own stream and frame k-1's pixels drain to the host. The members above (scene, ramps,
-    // atlas, layout, ..., h_bump) are the CURRENT slot; `other` holds the parked one and swap_slot() exchanges them.
-    struct SceneSlot {
-        DevBuf scene, ramps, atlas;
-        VbLayout layout{};
-        size_t scene_words = 0;
-        uint32_t n_ramps = 0, atlas_w = 0, atlas_h = 0;
-        bool have_scene = false;
-        VbBump *h_bump = nullptr, *h_bump_dev = nullptr;
-    } other;
-    uint32_t cur_slot = 0;
-    cudaStream_t upload_stream = nullptr;
-    cudaEvent_t upload_done[2]{}, raster_done[2]{};
-    struct RingFrame { // a streamed frame between vb_render_begin and its completion on the host
-        bool pending = false, raster_checked = false;
-        vb_params params{};
-        void *out_host = nullptr;
-        uint32_t slot = 0;
-        vb_frame_stats stats{};
-    } ring[3];
-    uint64_t stream_seq = 0;
-
-    // multi-GPU exchange (flatten sharded by tag range; k_exchange.cu)
-    struct Exchange {
-        bool configured = false, enabled = false;
-        uint32_t rank = 0, world = 1, lines_cap = 0, n_paths = 0;
-        size_t half_bytes = 0;
-        DevBuf arena;
-        void *peer[8] = {};
-        uint32_t rows[9] = {};
-    } xc;
-};
-
-static void swap_slot(vb_renderer *r) {
-    std::swap(r->scene, r->other.scene);
-    std::swap(r->ramps, r->other.ramps);
-    std::swap(r->atlas, r->other.atlas);
-    std::swap(r->layout, r->other.layout);
-    std::swap(r->scene_words, r->other.scene_words);
-    std::swap(r->n_ramps, r->other.n_ramps);
-    std::swap(r->atlas_w, r->other.atlas_w);
-    std::swap(r->atlas_h, r->other.atlas_h);
-    std::swap(r->have_scene, r->other.have_scene);
-    std::swap(r->h_bump, r->other.h_bump);
-    std::swap(r->h_bump_dev, r->other.h_bump_dev);
-    r->cur_slot ^= 1u;
-}
-static void select_slot(vb_renderer *r, uint32_t slot) {
-    if (r->cur_slot != slot) swap_slot(r);
-}
-
-#define CK(call)                                                                                  \
-    do {                                                                                          \
-        cudaError_t e_ = (call);                                                                  \
-        if (e_ != cudaSuccess) {                                                                  \
-            r->err = std::string(#call) + ": " + cudaGetErrorString(e_);                          \
-            return VB_E_CUDA;                                                                     \
-        }                                                                                         \
-    } while (0)
-
 static int ensure(vb_renderer *r, DevBuf &b, size_t bytes) {
     if (bytes < 256) bytes = 256;
     if (b.cap >= bytes) return VB_OK;
-    if (b.p) CK(cudaFree(b.p));
+    if (b.p) CK(r->err, cudaFree(b.p));
     b.p = nullptr;
     b.cap = 0;
     size_t want = (bytes + 255) & ~(size_t)255;
-    CK(cudaMalloc(&b.p, want));
+    CK(r->err, cudaMalloc(&b.p, want));
     b.cap = want;
     return VB_OK;
 }
+// Every device buffer of a renderer except the scene slots, resolve_tmp and the exchange arena: what vb_frame_stats.arena_bytes
+// counts (with both slots' scene, ramps and atlas). `key`: its address is part of a captured graph's key; the targets are
+// not, the frame's destination is.
+using BufMember = DevBuf vb_renderer::*;
+static const struct {
+    BufMember buf;
+    bool key;
+} kBuffers[] = {
+    {&vb_renderer::mask8, true},        {&vb_renderer::mask16, true},        {&vb_renderer::tag_monoids, true},
+    {&vb_renderer::path_bboxes, true},  {&vb_renderer::draw_monoids, true},  {&vb_renderer::info_bin_data, true},
+    {&vb_renderer::clip_inp, true},     {&vb_renderer::clip_bboxes, true},   {&vb_renderer::clip_scratch, true},
+    {&vb_renderer::draw_bboxes, true},  {&vb_renderer::bin_headers, true},   {&vb_renderer::paths, true},
+    {&vb_renderer::ctl, true},          {&vb_renderer::target, false},       {&vb_renderer::target_alt, false},
+    {&vb_renderer::tile_start, true},   {&vb_renderer::cls_list, true},      {&vb_renderer::lines, true},
+    {&vb_renderer::line_scratch, true}, {&vb_renderer::flatten_jobs, true},  {&vb_renderer::flatten_parts, true},
+    {&vb_renderer::tiles, true},        {&vb_renderer::seg_counts, true},    {&vb_renderer::segments, true},
+    {&vb_renderer::ptcl, true},         {&vb_renderer::blend_spill, true},
+};
+
 static size_t arena_bytes(const vb_renderer *r) {
-    const DevBuf *all[] = {&r->scene, &r->ramps, &r->atlas, &r->mask8, &r->mask16, &r->tag_monoids, &r->path_bboxes, &r->draw_monoids,
-                           &r->info_bin_data, &r->clip_inp, &r->clip_bboxes, &r->clip_scratch, &r->draw_bboxes, &r->bin_headers, &r->paths,
-                           &r->ctl, &r->target, &r->target_alt, &r->tile_start, &r->cls_list, &r->lines, &r->line_scratch, &r->flatten_jobs, &r->flatten_parts, &r->tiles, &r->seg_counts, &r->segments, &r->ptcl, &r->blend_spill};
-    size_t s = r->other.scene.cap + r->other.ramps.cap + r->other.atlas.cap;
-    for (auto b : all) s += b->cap;
+    size_t s = 0;
+    for (const SceneSlot &sl : r->slot) s += sl.scene.cap + sl.ramps.cap + sl.atlas.cap;
+    for (const auto &b : kBuffers) s += (r->*b.buf).cap;
     return s;
 }
 
@@ -316,25 +194,19 @@ extern "C" int vb_renderer_new(const vb_options *opt, vb_renderer **out) {
     cudaError_t e = cudaSetDevice(r->device);
     if (e != cudaSuccess) {
         fprintf(stderr, "vello_b200: cudaSetDevice(%d): %s\n", r->device, cudaGetErrorString(e));
-        delete r;
+        vb_renderer_free(r);
         return VB_E_CUDA;
     }
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, r->device) == cudaSuccess) r->sm_count = prop.multiProcessorCount;
-    if (cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaHostAlloc((void **)&r->h_bump, sizeof(VbBump), cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer((void **)&r->h_bump_dev, r->h_bump, 0) != cudaSuccess) {
-        delete r;
-        return VB_E_CUDA;
+    bool ok = cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking) == cudaSuccess &&
+              cudaStreamCreateWithFlags(&r->upload_stream, cudaStreamNonBlocking) == cudaSuccess &&
+              cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking) == cudaSuccess;
+    for (SceneSlot &s : r->slot) {
+        ok = ok && cudaHostAlloc((void **)&s.h_bump, sizeof(VbBump), cudaHostAllocMapped) == cudaSuccess &&
+             cudaHostGetDevicePointer((void **)&s.h_bump_dev, s.h_bump, 0) == cudaSuccess;
+        if (ok) memset(s.h_bump, 0, sizeof(VbBump));
     }
-    memset(r->h_bump, 0, sizeof(VbBump));
-    if (cudaHostAlloc((void **)&r->other.h_bump, sizeof(VbBump), cudaHostAllocMapped) != cudaSuccess ||
-        cudaHostGetDevicePointer((void **)&r->other.h_bump_dev, r->other.h_bump, 0) != cudaSuccess ||
-        cudaStreamCreateWithFlags(&r->upload_stream, cudaStreamNonBlocking) != cudaSuccess) {
-        delete r;
-        return VB_E_CUDA;
-    }
-    memset(r->other.h_bump, 0, sizeof(VbBump));
     for (auto &ev : r->upload_done) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     for (auto &ev : r->raster_done) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     for (auto &ev : r->ev) cudaEventCreate(&ev);
@@ -342,19 +214,10 @@ extern "C" int vb_renderer_new(const vb_options *opt, vb_renderer **out) {
     for (auto &ev : r->band_ev) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     for (auto &ev : r->copy_done) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     if (getenv("VELLO_B200_NO_GRAPH")) r->use_graph = false;
-    if (cudaStreamCreateWithFlags(&r->copy_stream, cudaStreamNonBlocking) != cudaSuccess) {
-        delete r;
-        return VB_E_CUDA;
-    }
-    r->ev_ok = true;
-    if (vb_fine_init_constants() != 0) {
-        delete r;
-        return VB_E_CUDA;
-    }
     std::vector<uint32_t> l8, l16;
     make_mask_luts(l8, l16);
-    if (ensure(r, r->mask8, l8.size() * 4) || ensure(r, r->mask16, l16.size() * 4)) {
-        delete r;
+    if (!ok || vb_fine_init_constants() != 0 || ensure(r, r->mask8, l8.size() * 4) || ensure(r, r->mask16, l16.size() * 4)) {
+        vb_renderer_free(r);
         return VB_E_CUDA;
     }
     cudaMemcpy(r->mask8.p, l8.data(), l8.size() * 4, cudaMemcpyHostToDevice);
@@ -363,32 +226,35 @@ extern "C" int vb_renderer_new(const vb_options *opt, vb_renderer **out) {
     return VB_OK;
 }
 
+template <size_t N> static void destroy_events(cudaEvent_t (&evs)[N]) {
+    for (cudaEvent_t ev : evs)
+        if (ev) cudaEventDestroy(ev);
+}
+
+// Also frees a partly built renderer (vb_renderer_new's error paths): whatever was not created is null.
 extern "C" void vb_renderer_free(vb_renderer *r) {
     if (!r) return;
     cudaSetDevice(r->device);
     if (r->stream) cudaStreamSynchronize(r->stream);
-    DevBuf *all[] = {&r->scene, &r->ramps, &r->atlas, &r->mask8, &r->mask16, &r->tag_monoids, &r->path_bboxes, &r->draw_monoids,
-                     &r->info_bin_data, &r->clip_inp, &r->clip_bboxes, &r->clip_scratch, &r->draw_bboxes, &r->bin_headers, &r->paths,
-                     &r->ctl, &r->target, &r->target_alt, &r->tile_start, &r->cls_list, &r->lines, &r->line_scratch, &r->flatten_jobs, &r->flatten_parts, &r->tiles, &r->seg_counts, &r->segments, &r->ptcl, &r->blend_spill};
-    for (auto b : all)
-        if (b->p) cudaFree(b->p);
-    for (DevBuf *b : {&r->other.scene, &r->other.ramps, &r->other.atlas, &r->resolve_tmp, &r->xc.arena})
-        if (b->p) cudaFree(b->p);
-    if (r->h_bump) cudaFreeHost(r->h_bump);
-    if (r->other.h_bump) cudaFreeHost(r->other.h_bump);
-    if (r->ev_ok) {
-        for (auto &ev : r->ev) cudaEventDestroy(ev);
-        for (auto &ev : r->frame_ev) cudaEventDestroy(ev);
-        for (auto &ev : r->band_ev) cudaEventDestroy(ev);
-        for (auto &ev : r->copy_done) cudaEventDestroy(ev);
-        for (auto &ev : r->upload_done) cudaEventDestroy(ev);
-        for (auto &ev : r->raster_done) cudaEventDestroy(ev);
-        for (auto &gs : r->graphs)
-            if (gs.exec) cudaGraphExecDestroy(gs.exec);
+    for (const auto &b : kBuffers)
+        if ((r->*b.buf).p) cudaFree((r->*b.buf).p);
+    for (SceneSlot &s : r->slot) {
+        for (DevBuf *b : {&s.scene, &s.ramps, &s.atlas})
+            if (b->p) cudaFree(b->p);
+        if (s.h_bump) cudaFreeHost(s.h_bump);
     }
-    if (r->copy_stream) cudaStreamDestroy(r->copy_stream);
-    if (r->upload_stream) cudaStreamDestroy(r->upload_stream);
-    if (r->stream) cudaStreamDestroy(r->stream);
+    for (DevBuf *b : {&r->resolve_tmp, &r->xc.arena})
+        if (b->p) cudaFree(b->p);
+    destroy_events(r->ev);
+    destroy_events(r->frame_ev);
+    destroy_events(r->band_ev);
+    destroy_events(r->copy_done);
+    destroy_events(r->upload_done);
+    destroy_events(r->raster_done);
+    for (auto &gs : r->graphs)
+        if (gs.exec) cudaGraphExecDestroy(gs.exec);
+    for (cudaStream_t st : {r->copy_stream, r->upload_stream, r->stream})
+        if (st) cudaStreamDestroy(st);
     delete r;
 }
 
@@ -412,40 +278,37 @@ extern "C" void *vb_target(vb_renderer *r, size_t *bytes) {
 }
 extern "C" int vb_copy_to_host(vb_renderer *r, const void *src_device, void *dst_host, size_t bytes) {
     if (!r || !src_device || !dst_host) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaMemcpyAsync(dst_host, src_device, bytes, cudaMemcpyDeviceToHost, r->stream));
-    CK(cudaStreamSynchronize(r->stream));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaMemcpyAsync(dst_host, src_device, bytes, cudaMemcpyDeviceToHost, r->stream));
+    CK(r->err, cudaStreamSynchronize(r->stream));
     return VB_OK;
 }
 
-static int upload_on(vb_renderer *r, cudaStream_t st, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
-                     uint32_t ramp_w, uint32_t ramp_h, const uint8_t *atlas, uint32_t atlas_w, uint32_t atlas_h) {
+int upload_on(vb_renderer *r, cudaStream_t st, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
+              uint32_t ramp_w, uint32_t ramp_h, const uint8_t *atlas, uint32_t atlas_w, uint32_t atlas_h) {
     if (!r || !layout || (scene_len && !scene) || (scene_len & 3)) return VB_E_INVALID;
     if (ramp_h && ramp_w != 512) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    memcpy(&r->layout, layout, sizeof(VbLayout));
-    r->scene_words = scene_len / 4;
+    CK(r->err, cudaSetDevice(r->device));
+    SceneSlot &s = r->cur();
+    memcpy(&s.layout, layout, sizeof(VbLayout));
+    s.scene_words = scene_len / 4;
     int rc;
-    if ((rc = ensure(r, r->scene, scene_len + 64))) return rc;
-    if (scene_len) CK(cudaMemcpyAsync(r->scene.p, scene, scene_len, cudaMemcpyHostToDevice, st));
-    r->n_ramps = ramp_h;
-    if ((rc = ensure(r, r->ramps, (size_t)ramp_h * 512 * 4))) return rc;
-    if (ramp_h) CK(cudaMemcpyAsync(r->ramps.p, ramps, (size_t)ramp_h * 512 * 4, cudaMemcpyHostToDevice, st));
-    r->atlas_w = atlas ? atlas_w : 0;
-    r->atlas_h = atlas ? atlas_h : 0;
-    if ((rc = ensure(r, r->atlas, (size_t)r->atlas_w * r->atlas_h * 4))) return rc;
-    if (r->atlas_w && r->atlas_h)
-        CK(cudaMemcpyAsync(r->atlas.p, atlas, (size_t)r->atlas_w * r->atlas_h * 4, cudaMemcpyHostToDevice, st));
-    r->have_scene = true;
+    if ((rc = ensure(r, s.scene, scene_len + 64))) return rc;
+    if (scene_len) CK(r->err, cudaMemcpyAsync(s.scene.p, scene, scene_len, cudaMemcpyHostToDevice, st));
+    s.n_ramps = ramp_h;
+    if ((rc = ensure(r, s.ramps, (size_t)ramp_h * 512 * 4))) return rc;
+    if (ramp_h) CK(r->err, cudaMemcpyAsync(s.ramps.p, ramps, (size_t)ramp_h * 512 * 4, cudaMemcpyHostToDevice, st));
+    s.atlas_w = atlas ? atlas_w : 0;
+    s.atlas_h = atlas ? atlas_h : 0;
+    if ((rc = ensure(r, s.atlas, (size_t)s.atlas_w * s.atlas_h * 4))) return rc;
+    if (s.atlas_w && s.atlas_h)
+        CK(r->err, cudaMemcpyAsync(s.atlas.p, atlas, (size_t)s.atlas_w * s.atlas_h * 4, cudaMemcpyHostToDevice, st));
+    s.have_scene = true;
     return VB_OK;
 }
 
-extern "C" int vb_readback_wait(vb_renderer *r);
-// A non-streaming entry point used while streamed frames are still in flight completes them first.
-static int drain_stream(vb_renderer *r) {
-    if (r->stream_pending && !r->in_stream_call) return vb_readback_wait(r);
-    return VB_OK;
-}
+// A public entry point other than the streaming pair, used while streamed frames are still in flight, completes them first.
+static int drain_stream(vb_renderer *r) { return r->stream_pending ? vb_readback_wait(r) : VB_OK; }
 
 extern "C" int vb_scene_upload(vb_renderer *r, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
                                uint32_t ramp_w, uint32_t ramp_h, const uint8_t *atlas, uint32_t atlas_w, uint32_t atlas_h) {
@@ -481,7 +344,8 @@ static int prepare(vb_renderer *r, const vb_params *p) {
     c.target_width = p->width;
     c.target_height = p->height;
     c.base_color = p->base_color;
-    c.layout = r->layout;
+    const SceneSlot &s = r->cur();
+    c.layout = s.layout;
     const uint32_t hb = (c.height_in_tiles + 15u) / 16u, wb = (c.width_in_tiles + 15u) / 16u;
     c.win_by0 = 0;
     c.win_by1 = hb;
@@ -500,16 +364,16 @@ static int prepare(vb_renderer *r, const vb_params *p) {
         c.win_by1 = (c.win_ty1 + 15u) / 16u;
     }
     c.win_cull = (c.win_ty0 > 0u || c.win_ty1 < c.height_in_tiles) ? 1u : 0u;
-    c.n_tag_words = r->layout.path_data_base - r->layout.path_tag_base;
-    c.scene_words = (uint32_t)r->scene_words;
-    c.n_ramps = r->n_ramps;
-    c.atlas_w = r->atlas_w;
-    c.atlas_h = r->atlas_h;
+    c.n_tag_words = s.layout.path_data_base - s.layout.path_tag_base;
+    c.scene_words = (uint32_t)s.scene_words;
+    c.n_ramps = s.n_ramps;
+    c.atlas_w = s.atlas_w;
+    c.atlas_h = s.atlas_h;
     c.out_pitch_px = p->width;
     c.out_row0 = c.win_ty0 * 16u;
     r->params = *p;
 
-    const VbLayout &L = r->layout;
+    const VbLayout &L = s.layout;
     const uint32_t n_draw = L.n_draw_objects, n_paths = L.n_paths, n_clips = L.n_clips;
     const uint32_t n_tiles = c.width_in_tiles * c.height_in_tiles;
     const uint32_t n_bins = wb * hb, aligned_n_bins = (n_bins + 255u) & ~255u;
@@ -591,9 +455,29 @@ static void rec(vb_renderer *r, int i) {
     if (r->timing) cudaEventRecord(r->ev[i], r->stream);
 }
 
-// Enqueue stages first..last. Does not synchronise.
-static int enqueue_direct(vb_renderer *r, int first, int last, void *out_dev) {
+// grid of the kernels that stride over a bump arena: from its capacity, at most 16 blocks per SM
+static uint32_t arena_grid(const vb_renderer *r, uint32_t cap) {
+    const uint64_t blocks = ((uint64_t)cap + 255) / 256;
+    return (uint32_t)(blocks < (uint64_t)r->sm_count * 16 ? blocks : (uint64_t)r->sm_count * 16);
+}
+
+// Queue the device->host copy of the destination's tile rows ty0..ty1 on copy_stream, behind what `stream` has enqueued so far.
+static int queue_readback(vb_renderer *r, const FrameDest &d, uint32_t ty0, uint32_t ty1, uint32_t band) {
     const VbConfig &c = r->cfg;
+    size_t y0 = (size_t)ty0 * 16u, y1 = (size_t)ty1 * 16u;
+    if (y1 > c.target_height) y1 = c.target_height;
+    if (y1 <= y0) return VB_OK;
+    const size_t off = (y0 - c.out_row0) * c.out_pitch_px * 4u, bytes = (y1 - y0) * c.out_pitch_px * 4u;
+    CK(r->err, cudaEventRecord(r->band_ev[band], r->stream));
+    CK(r->err, cudaStreamWaitEvent(r->copy_stream, r->band_ev[band], 0));
+    CK(r->err, cudaMemcpyAsync((char *)d.host_out + off, (const char *)d.out_dev + off, bytes, cudaMemcpyDeviceToHost, r->copy_stream));
+    return VB_OK;
+}
+
+// Enqueue stages first..last. Does not synchronise.
+static int enqueue_direct(vb_renderer *r, int first, int last, const FrameDest &d) {
+    const VbConfig &c = r->cfg;
+    const SceneSlot &s = r->cur();
     cudaStream_t st = r->stream;
     uint32_t *ctl = (uint32_t *)r->ctl.p;
     VbBump *bump = (VbBump *)ctl;
@@ -608,44 +492,45 @@ static int enqueue_direct(vb_renderer *r, int first, int last, void *out_dev) {
                                                              xepoch);
         launches++;
     }
-    else if (r->zero_fine_queue) {
+    else if (d.zero_fine_queue) {
         // vb_run_stages starting after stage 0: the control block is not zeroed, but fine's tile queues must start at 0 and
         // coarse must append to empty class lists
-        if (last >= VB_STAGE_ID_FINE) CK(cudaMemsetAsync(ctl + VB_CTL_FINE_QUEUE, 0, 8 * sizeof(uint32_t), st));
+        if (last >= VB_STAGE_ID_FINE) CK(r->err, cudaMemsetAsync(ctl + VB_CTL_FINE_QUEUE, 0, 8 * sizeof(uint32_t), st));
         if (first <= VB_STAGE_ID_COARSE && last >= VB_STAGE_ID_COARSE)
-            CK(cudaMemsetAsync(ctl + VB_CTL_FINE_CLASS, 0, VB_FINE_CLASSES * sizeof(uint32_t), st));
+            CK(r->err, cudaMemsetAsync(ctl + VB_CTL_FINE_CLASS, 0, VB_FINE_CLASSES * sizeof(uint32_t), st));
     }
     rec(r, 0);
-    for (int s = first; s <= last; s++) {
-        switch (s) {
+    for (int stage = first; stage <= last; stage++) {
+        switch (stage) {
         case VB_STAGE_ID_PATHTAG:
-            vb_launch_pathtag(&c, (const uint32_t *)r->scene.p, (VbTagMonoid *)r->tag_monoids.p, ctl + r->off_lb_pathtag, r->parts_pathtag, st);
+            vb_launch_pathtag(&c, (const uint32_t *)s.scene.p, (VbTagMonoid *)r->tag_monoids.p, ctl + r->off_lb_pathtag, r->parts_pathtag, st);
             launches += r->parts_pathtag ? 1 : 0;
             break;
-        case VB_STAGE_ID_FLATTEN:
+        case VB_STAGE_ID_FLATTEN: {
+            // With the exchange on, this GPU flattens its share of the tag stream (no stripe culling: the lines are for
+            // everybody), then the lines and path boxes are exchanged through peer memory (k_exchange.cu).
+            VbConfig cf = c;
+            uint32_t p0 = 0u, p1 = r->parts_flatten;
             if (r->xc.enabled) {
-                // this GPU flattens its share of the tag stream (no stripe culling: the lines are for everybody), then the
-                // lines and path boxes are exchanged through peer memory (k_exchange.cu)
-                VbConfig cx = c;
-                cx.win_cull = 0u;
                 const uint32_t P = r->parts_flatten, G = r->xc.world, k = r->xc.rank;
-                const uint32_t p0 = (uint32_t)((uint64_t)P * k / G) & ~7u;
-                const uint32_t p1 = k + 1u == G ? P : ((uint32_t)((uint64_t)P * (k + 1u) / G) & ~7u);
-                vb_launch_flatten(&cx, (const uint32_t *)r->scene.p, (const VbTagMonoid *)r->tag_monoids.p, (VbPathBbox *)r->path_bboxes.p, bump,
-                                  (VbLineSoup *)r->lines.p, r->line_scratch.p, r->flatten_jobs.p, (uint32_t *)r->flatten_parts.p,
-                                  ctl + r->off_lb_flatten, r->parts_flatten, first != 0 ? 1 : 0, p0, p1, st);
+                cf.win_cull = 0u;
+                p0 = (uint32_t)((uint64_t)P * k / G) & ~7u;
+                p1 = k + 1u == G ? P : ((uint32_t)((uint64_t)P * (k + 1u) / G) & ~7u);
+            }
+            vb_launch_flatten(&cf, (const uint32_t *)s.scene.p, (const VbTagMonoid *)r->tag_monoids.p, (VbPathBbox *)r->path_bboxes.p, bump,
+                              (VbLineSoup *)r->lines.p, r->line_scratch.p, r->flatten_jobs.p, (uint32_t *)r->flatten_parts.p,
+                              ctl + r->off_lb_flatten, r->parts_flatten, first != 0 ? 1 : 0, p0, p1, st);
+            if (r->xc.enabled) {
                 XPeersHost X;
                 xpeers_of(r, &X);
                 vb_launch_exchange_send(&X, bump, c.lines_size, (VbLineSoup *)r->lines.p, ctl + VB_CTL_XCHG_SCRATCH,
                                         (VbPathBbox *)r->path_bboxes.p, r->sm_count, st);
                 launches += (r->parts_flatten ? 3 : 0) + 4;
-                break;
+            } else {
+                launches += (first != 0 && c.layout.n_paths ? 1 : 0) + (r->parts_flatten ? 3 : 0);
             }
-            vb_launch_flatten(&c, (const uint32_t *)r->scene.p, (const VbTagMonoid *)r->tag_monoids.p, (VbPathBbox *)r->path_bboxes.p, bump,
-                              (VbLineSoup *)r->lines.p, r->line_scratch.p, r->flatten_jobs.p, (uint32_t *)r->flatten_parts.p,
-                              ctl + r->off_lb_flatten, r->parts_flatten, first != 0 ? 1 : 0, 0u, r->parts_flatten, st);
-            launches += (first != 0 && c.layout.n_paths ? 1 : 0) + (r->parts_flatten ? 3 : 0);
             break;
+        }
         case VB_STAGE_ID_DRAW:
             if (r->xc.enabled) { // second half of the exchange: my lines and the complete path boxes arrive before draw_leaf reads them
                 XPeersHost X;
@@ -653,7 +538,7 @@ static int enqueue_direct(vb_renderer *r, int first, int last, void *out_dev) {
                 vb_launch_exchange_recv(&X, bump, c.lines_size, (VbLineSoup *)r->lines.p, (VbPathBbox *)r->path_bboxes.p, r->sm_count, st);
                 launches += 3;
             }
-            vb_launch_draw(&c, (const uint32_t *)r->scene.p, (const VbPathBbox *)r->path_bboxes.p, (VbDrawMonoid *)r->draw_monoids.p,
+            vb_launch_draw(&c, (const uint32_t *)s.scene.p, (const VbPathBbox *)r->path_bboxes.p, (VbDrawMonoid *)r->draw_monoids.p,
                            (uint32_t *)r->info_bin_data.p, (VbClipInp *)r->clip_inp.p, ctl + r->off_lb_draw, r->parts_draw, st);
             launches += r->parts_draw ? 1 : 0;
             break;
@@ -670,43 +555,37 @@ static int enqueue_direct(vb_renderer *r, int first, int last, void *out_dev) {
             launches += n_draw ? 1 : 0;
             break;
         case VB_STAGE_ID_TILE_ALLOC:
-            vb_launch_tile_alloc(&c, (const uint32_t *)r->scene.p, (const VbBbox4 *)r->draw_bboxes.p, bump, (VbPath *)r->paths.p,
+            vb_launch_tile_alloc(&c, (const uint32_t *)s.scene.p, (const VbBbox4 *)r->draw_bboxes.p, bump, (VbPath *)r->paths.p,
                                  (VbTile *)r->tiles.p, ctl + r->off_lb_tile, r->parts_tile, st);
             launches += r->parts_tile ? 2 : 0;
             break;
-        case VB_STAGE_ID_PATH_COUNT: {
-            // grid from the arena capacity; the kernel strides over bump.lines read on the device
-            uint64_t blocks = ((uint64_t)c.lines_size + 255) / 256;
-            uint32_t grid = (uint32_t)(blocks < (uint64_t)r->sm_count * 16 ? blocks : (uint64_t)r->sm_count * 16);
+        case VB_STAGE_ID_PATH_COUNT: // the kernel strides over bump.lines read on the device
             vb_launch_path_count(&c, bump, (const VbLineSoup *)r->lines.p, (const VbPath *)r->paths.p, (VbTile *)r->tiles.p,
-                                 (VbSegmentCount *)r->seg_counts.p, grid, st);
+                                 (VbSegmentCount *)r->seg_counts.p, arena_grid(r, c.lines_size), st);
             launches += 1;
             break;
-        }
         case VB_STAGE_ID_BACKDROP:
             vb_launch_backdrop(&c, bump, (const VbPath *)r->paths.p, (VbTile *)r->tiles.p, st);
             launches += n_draw ? 1 : 0;
             break;
         case VB_STAGE_ID_COARSE:
-            vb_launch_coarse(&c, (const uint32_t *)r->scene.p, (const VbDrawMonoid *)r->draw_monoids.p, (const VbBinHeader *)r->bin_headers.p,
+            vb_launch_coarse(&c, (const uint32_t *)s.scene.p, (const VbDrawMonoid *)r->draw_monoids.p, (const VbBinHeader *)r->bin_headers.p,
                              (const uint32_t *)r->info_bin_data.p, (const VbPath *)r->paths.p, (VbTile *)r->tiles.p, bump,
                              (uint32_t *)r->ptcl.p, (uint32_t *)r->tile_start.p, r->cls_list.p, c.width_in_tiles * c.height_in_tiles, st);
             launches += 1;
             break;
-        case VB_STAGE_ID_PATH_TILING: {
-            uint64_t blocks = ((uint64_t)c.seg_counts_size + 255) / 256;
-            uint32_t grid = (uint32_t)(blocks < (uint64_t)r->sm_count * 16 ? blocks : (uint64_t)r->sm_count * 16);
+        case VB_STAGE_ID_PATH_TILING:
             vb_launch_path_tiling(&c, bump, (const VbSegmentCount *)r->seg_counts.p, (const VbLineSoup *)r->lines.p,
-                                  (const VbPath *)r->paths.p, (const VbTile *)r->tiles.p, (VbSegment *)r->segments.p, grid, st);
+                                  (const VbPath *)r->paths.p, (const VbTile *)r->tiles.p, (VbSegment *)r->segments.p,
+                                  arena_grid(r, c.seg_counts_size), st);
             launches += 1;
             break;
-        }
         case VB_STAGE_ID_FINE: {
-            // With a host destination (vb_render) fine is launched in up to 8 bands of tile rows and each band's
-            // device->host copy is queued on a second stream behind an event, so the read-back of band k overlaps
-            // the rasterisation of band k+1 (only the last band's copy is exposed).
+            // With a host destination fine is launched in up to d.bands bands of tile rows and each band's device->host copy
+            // is queued on a second stream behind an event, so the read-back of band k overlaps the rasterisation of band
+            // k+1 (only the last band's copy is exposed).
             const uint32_t rows = c.win_ty1 - c.win_ty0;
-            uint32_t n_bands = (r->host_out && rows >= 64u) ? r->readback_bands : 1u;
+            const uint32_t n_bands = (d.host_out && rows >= 64u) ? d.bands : 1u;
             const uint32_t band_rows = (rows + n_bands - 1u) / n_bands;
             for (uint32_t b = 0; b < n_bands; b++) {
                 VbConfig cb = c;
@@ -714,32 +593,26 @@ static int enqueue_direct(vb_renderer *r, int first, int last, void *out_dev) {
                 cb.win_ty1 = cb.win_ty0 + band_rows < c.win_ty1 ? cb.win_ty0 + band_rows : c.win_ty1;
                 if (cb.win_ty0 >= cb.win_ty1) break;
                 vb_launch_fine(&cb, (int)r->params.aa, bump, (const VbSegment *)r->segments.p, (const uint32_t *)r->ptcl.p,
-                               (const uint32_t *)r->info_bin_data.p, (uint32_t *)r->blend_spill.p, (uint32_t *)out_dev,
-                               (const uint32_t *)r->ramps.p, (const uint8_t *)r->atlas.p, (const uint32_t *)r->mask8.p,
+                               (const uint32_t *)r->info_bin_data.p, (uint32_t *)r->blend_spill.p, (uint32_t *)d.out_dev,
+                               (const uint32_t *)s.ramps.p, (const uint8_t *)s.atlas.p, (const uint32_t *)r->mask8.p,
                                (const uint32_t *)r->mask16.p, (const uint32_t *)r->tile_start.p, r->occlusion_cull,
                                ctl + VB_CTL_FINE_QUEUE + b, r->cls_list.p, n_bands == 1u ? ctl + VB_CTL_FINE_CLASS : nullptr,
                                c.width_in_tiles * c.height_in_tiles, r->sm_count, st);
                 launches += 1;
-                if (r->host_out) {
-                    size_t y0 = (size_t)cb.win_ty0 * 16u, y1 = (size_t)cb.win_ty1 * 16u;
-                    if (y1 > c.target_height) y1 = c.target_height;
-                    if (y1 > y0) {
-                        const size_t off = (y0 - c.out_row0) * c.out_pitch_px * 4u, bytes = (y1 - y0) * c.out_pitch_px * 4u;
-                        CK(cudaEventRecord(r->band_ev[b], st));
-                        CK(cudaStreamWaitEvent(r->copy_stream, r->band_ev[b], 0));
-                        CK(cudaMemcpyAsync((char *)r->host_out + off, (const char *)out_dev + off, bytes, cudaMemcpyDeviceToHost, r->copy_stream));
-                    }
+                if (d.host_out) {
+                    const int rc = queue_readback(r, d, cb.win_ty0, cb.win_ty1, b);
+                    if (rc) return rc;
                 }
             }
             break;
         }
         default: return VB_E_INVALID;
         }
-        rec(r, s + 1);
+        rec(r, stage + 1);
     }
-    k_publish_bump<<<1, 32, 0, st>>>(bump, r->h_bump_dev); // zero-copy store to mapped host memory (no copy engine)
+    k_publish_bump<<<1, 32, 0, st>>>(bump, s.h_bump_dev); // zero-copy store to mapped host memory (no copy engine)
     launches++;
-    CK(cudaGetLastError());
+    CK(r->err, cudaGetLastError());
     r->launches = launches;
     return VB_OK;
 }
@@ -751,17 +624,16 @@ static int enqueue_direct(vb_renderer *r, int first, int last, void *out_dev) {
 // the launches of a frame are identical -- same kernels, grids, arena pointers, config -- so they are captured once into a
 // graph and replayed with ONE submission. The key is everything a launch argument is derived from; growing an arena or
 // changing the scene layout / frame size / window simply misses the cache and re-captures.
-static void graph_key(const vb_renderer *r, int last, const void *out_dev, GraphKey *k) {
+static void graph_key(vb_renderer *r, int last, const void *out_dev, GraphKey *k) {
     memset(k, 0, sizeof *k);
     k->cfg = r->cfg;
-    const DevBuf *bufs[] = {&r->scene, &r->ramps, &r->atlas, &r->mask8, &r->mask16, &r->tag_monoids, &r->path_bboxes, &r->draw_monoids,
-                            &r->info_bin_data, &r->clip_inp, &r->clip_bboxes, &r->clip_scratch, &r->draw_bboxes, &r->bin_headers, &r->paths,
-                            &r->ctl, &r->tile_start, &r->cls_list, &r->lines, &r->line_scratch, &r->flatten_jobs, &r->flatten_parts, &r->tiles,
-                            &r->seg_counts, &r->segments, &r->ptcl, &r->blend_spill};
+    const SceneSlot &s = r->cur();
     size_t n = 0;
-    for (const DevBuf *b : bufs) k->ptrs[n++] = b->p;
+    for (const DevBuf *b : {&s.scene, &s.ramps, &s.atlas}) k->ptrs[n++] = b->p;
+    for (const auto &b : kBuffers)
+        if (b.key) k->ptrs[n++] = (r->*b.buf).p;
     k->ptrs[n++] = out_dev;
-    k->ptrs[n++] = r->h_bump_dev;
+    k->ptrs[n++] = s.h_bump_dev;
     k->ctl_words = r->ctl_words;
     k->aa = r->params.aa;
     k->cull = r->occlusion_cull;
@@ -773,62 +645,47 @@ static void graph_key(const vb_renderer *r, int last, const void *out_dev, Graph
     }
 }
 
-static int queue_readback(vb_renderer *r, const VbConfig &c, uint32_t ty0, uint32_t ty1, void *out_dev, uint32_t band) {
-    size_t y0 = (size_t)ty0 * 16u, y1 = (size_t)ty1 * 16u;
-    if (y1 > c.target_height) y1 = c.target_height;
-    if (y1 <= y0) return VB_OK;
-    const size_t off = (y0 - c.out_row0) * c.out_pitch_px * 4u, bytes = (y1 - y0) * c.out_pitch_px * 4u;
-    CK(cudaEventRecord(r->band_ev[band], r->stream));
-    CK(cudaStreamWaitEvent(r->copy_stream, r->band_ev[band], 0));
-    CK(cudaMemcpyAsync((char *)r->host_out + off, (const char *)out_dev + off, bytes, cudaMemcpyDeviceToHost, r->copy_stream));
-    return VB_OK;
-}
-
 // Enqueue stages first..last: through a cached graph for whole frames, directly otherwise.
-static int enqueue(vb_renderer *r, int first, int last, void *out_dev) {
+static int enqueue(vb_renderer *r, int first, int last, const FrameDest &d) {
     const VbConfig &c = r->cfg;
-    if (!r->use_graph || r->timing || first != 0 || last != VB_N_STAGE_IDS - 1) return enqueue_direct(r, first, last, out_dev);
+    if (!r->use_graph || r->timing || first != 0 || last != VB_N_STAGE_IDS - 1) return enqueue_direct(r, first, last, d);
     // with a host destination split into bands, fine and its interleaved copies stay outside the graph
     const uint32_t rows = c.win_ty1 - c.win_ty0;
-    const bool banded = r->host_out && rows >= 64u && r->readback_bands > 1u;
+    const bool banded = d.host_out && rows >= 64u && d.bands > 1u;
     const int g_last = banded ? VB_STAGE_ID_FINE - 1 : last;
     GraphKey key;
-    graph_key(r, g_last, out_dev, &key);
+    graph_key(r, g_last, d.out_dev, &key);
     GraphSlot *slot = nullptr;
     for (GraphSlot &gs : r->graphs)
         if (gs.exec && memcmp(&gs.key, &key, sizeof key) == 0) slot = &gs;
-    void *host_out = r->host_out;
+    // Any refusal along the way (a tool or driver that does not allow capture here) turns graph replay off for this renderer
+    // and the frame is launched kernel by kernel: graphs are an optimisation, never a requirement.
+    auto without_graph = [&]() {
+        cudaGetLastError();
+        r->use_graph = false;
+        return enqueue_direct(r, first, last, d);
+    };
     if (!slot) {
         slot = &r->graphs[r->graph_next++ % (sizeof r->graphs / sizeof r->graphs[0])];
         if (slot->exec) {
             cudaGraphExecDestroy(slot->exec);
             slot->exec = nullptr;
         }
-        // Any refusal along the way (a tool or driver that does not allow capture here) turns graph replay off for this
-        // renderer and the frame is launched kernel by kernel: graphs are an optimisation, never a requirement.
-        if (cudaStreamBeginCapture(r->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) {
-            cudaGetLastError();
-            r->use_graph = false;
-            return enqueue_direct(r, first, last, out_dev);
-        }
-        r->host_out = nullptr; // the captured fine is one launch; its read-back is queued after the graph, below
-        const int rc = enqueue_direct(r, 0, g_last, out_dev);
+        if (cudaStreamBeginCapture(r->stream, cudaStreamCaptureModeThreadLocal) != cudaSuccess) return without_graph();
+        FrameDest captured = d;
+        captured.host_out = nullptr; // the captured fine is one launch; its read-back is queued after the graph, below
+        const int rc = enqueue_direct(r, 0, g_last, captured);
         cudaGraph_t g = nullptr;
         const cudaError_t e = cudaStreamEndCapture(r->stream, &g);
-        r->host_out = host_out;
         if (rc != VB_OK || e != cudaSuccess || !g) {
             if (g) cudaGraphDestroy(g);
-            cudaGetLastError();
-            r->use_graph = false;
-            return enqueue_direct(r, first, last, out_dev);
+            return without_graph();
         }
         const cudaError_t ei = cudaGraphInstantiate(&slot->exec, g, 0);
         cudaGraphDestroy(g);
         if (ei != cudaSuccess) {
             slot->exec = nullptr;
-            cudaGetLastError();
-            r->use_graph = false;
-            return enqueue_direct(r, first, last, out_dev);
+            return without_graph();
         }
         slot->key = key;
         slot->launches = r->launches;
@@ -837,85 +694,73 @@ static int enqueue(vb_renderer *r, int first, int last, void *out_dev) {
         cudaGetLastError();
         cudaGraphExecDestroy(slot->exec);
         slot->exec = nullptr;
-        r->use_graph = false;
-        return enqueue_direct(r, first, last, out_dev);
+        return without_graph();
     }
     r->launches = slot->launches;
     if (banded) {
-        const int rc = enqueue_direct(r, VB_STAGE_ID_FINE, VB_STAGE_ID_FINE, out_dev);
+        const int rc = enqueue_direct(r, VB_STAGE_ID_FINE, VB_STAGE_ID_FINE, d);
         r->launches += slot->launches;
         return rc;
     }
-    if (host_out) return queue_readback(r, c, c.win_ty0, c.win_ty1, out_dev, 0);
+    if (d.host_out) return queue_readback(r, d, c.win_ty0, c.win_ty1, 0);
     return VB_OK;
 }
 
-static int pick_out(vb_renderer *r, void *out_device, void **out) {
-    if (out_device) {
-        *out = out_device;
-        return VB_OK;
-    }
+// Resolve a destination without a device buffer to the renderer's target, sized for the configured window.
+static int pick_out(vb_renderer *r, FrameDest &d) {
+    if (d.out_dev) return VB_OK;
     const VbConfig &c = r->cfg;
     size_t rows = (size_t)(c.win_ty1 - c.win_ty0) * 16u;
-    DevBuf &t = r->use_alt ? r->target_alt : r->target;
+    DevBuf &t = d.target ? r->target_alt : r->target;
     int rc = ensure(r, t, (size_t)c.out_pitch_px * 4u * rows);
-    *out = t.p;
+    d.out_dev = t.p;
     return rc;
 }
 
-// A frame is enqueued in two steps: everything that may allocate, free or otherwise synchronise with the device (config,
-// arenas, the output target), then the launches. vb_group runs step 1 for ALL its renderers before step 2 of any: with the
-// exchange on, a renderer's frame contains a kernel that waits for its peers, and a peer that shares the device (tests)
-// must not be stuck in a cudaFree behind that kernel.
-static int frame_prepare(vb_renderer *r, const vb_params *p, void *out_device) {
+int frame_prepare(vb_renderer *r, const vb_params *p, const FrameDest &d) {
     if (!r || !p) return VB_E_INVALID;
-    if (!r->have_scene) return VB_E_NO_SCENE;
-    CK(cudaSetDevice(r->device));
+    if (!r->cur().have_scene) return VB_E_NO_SCENE;
+    CK(r->err, cudaSetDevice(r->device));
+    FrameDest dest = d;
     int rc = prepare(r, p);
-    if (rc) return rc;
-    void *out;
-    if ((rc = pick_out(r, out_device, &out))) return rc;
-    r->out_dev = out;
-    return VB_OK;
+    if (rc == VB_OK) rc = pick_out(r, dest);
+    if (rc == VB_OK) r->dest = dest;
+    return rc;
 }
-static int frame_launch(vb_renderer *r) {
-    CK(cudaSetDevice(r->device));
-    CK(cudaEventRecord(r->frame_ev[0], r->stream));
-    int rc = enqueue(r, 0, VB_N_STAGE_IDS - 1, r->out_dev);
-    if (rc == VB_OK) CK(cudaEventRecord(r->frame_ev[1], r->stream));
+int frame_launch(vb_renderer *r) {
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaEventRecord(r->frame_ev[0], r->stream));
+    int rc = enqueue(r, 0, VB_N_STAGE_IDS - 1, r->dest);
+    if (rc == VB_OK) CK(r->err, cudaEventRecord(r->frame_ev[1], r->stream));
     r->frame_timed = rc == VB_OK;
-    r->frame_pending = rc == VB_OK;
     return rc;
 }
 
-// The same frame in two submissions (plain launches): up to and including flatten + the sending half of the exchange, then
-// the rest. Used by vb_group when renderers share a device, see k_exchange.cu.
-static int frame_launch_half(vb_renderer *r, int half) {
-    CK(cudaSetDevice(r->device));
+int frame_launch_half(vb_renderer *r, int half) {
+    CK(r->err, cudaSetDevice(r->device));
     if (half == 0) {
-        CK(cudaEventRecord(r->frame_ev[0], r->stream));
-        return enqueue_direct(r, 0, VB_STAGE_ID_FLATTEN, r->out_dev);
+        CK(r->err, cudaEventRecord(r->frame_ev[0], r->stream));
+        return enqueue_direct(r, 0, VB_STAGE_ID_FLATTEN, r->dest);
     }
     uint32_t first_half = r->launches;
-    int rc = enqueue_direct(r, VB_STAGE_ID_DRAW, VB_N_STAGE_IDS - 1, r->out_dev);
+    int rc = enqueue_direct(r, VB_STAGE_ID_DRAW, VB_N_STAGE_IDS - 1, r->dest);
     r->launches += first_half;
     // (with a host destination enqueue_direct queues the read-back behind fine itself)
-    if (rc == VB_OK) CK(cudaEventRecord(r->frame_ev[1], r->stream));
+    if (rc == VB_OK) CK(r->err, cudaEventRecord(r->frame_ev[1], r->stream));
     r->frame_timed = rc == VB_OK;
-    r->frame_pending = rc == VB_OK;
     return rc;
 }
 
 extern "C" int vb_render_enqueue(vb_renderer *r, const vb_params *p, void *out_device) {
-    int rc = frame_prepare(r, p, out_device);
+    int rc = frame_prepare(r, p, FrameDest{out_device, nullptr, 1u, 0u, false});
     if (rc) return rc;
     return frame_launch(r);
 }
 
-static void fill_stats(vb_renderer *r, vb_frame_stats *s) {
+void fill_stats(vb_renderer *r, vb_frame_stats *s) {
     if (!s) return;
     memset(s, 0, sizeof *s);
-    memcpy(s, r->h_bump, sizeof(VbBump));
+    memcpy(s, r->cur().h_bump, sizeof(VbBump));
     s->retries = r->retries;
     s->kernel_launches = r->launches;
     s->arena_bytes = arena_bytes(r);
@@ -925,9 +770,8 @@ static void fill_stats(vb_renderer *r, vb_frame_stats *s) {
     }
 }
 
-// After a failed attempt: enlarge whatever overflowed, using the counters the kernels kept counting.
-static void grow_arenas(vb_renderer *r) {
-    const VbBump &b = *r->h_bump;
+void grow_arenas(vb_renderer *r) {
+    const VbBump &b = *r->cur().h_bump;
     const VbConfig &c = r->cfg;
     if (b.lines > r->cap_lines) r->cap_lines = grow(b.lines);
     if (b.binning > r->cap_binning) r->cap_binning = grow(b.binning);
@@ -943,61 +787,59 @@ static void grow_arenas(vb_renderer *r) {
 
 extern "C" int vb_frame_finish(vb_renderer *r, vb_frame_stats *stats) {
     if (!r) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
-    r->frame_pending = false;
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
     fill_stats(r, stats);
-    return r->h_bump->failed ? VB_E_BUMP_OVERFLOW : VB_OK;
+    return r->cur().h_bump->failed ? VB_E_BUMP_OVERFLOW : VB_OK;
+}
+
+int wait_copies(vb_renderer *r, int rc) {
+    const cudaError_t e = cudaStreamSynchronize(r->copy_stream);
+    if (rc == VB_OK && e != cudaSuccess) {
+        r->err = std::string("copy stream: ") + cudaGetErrorString(e);
+        return VB_E_CUDA;
+    }
+    return rc;
+}
+
+int render_attempts(vb_renderer *r, const vb_params *p, const FrameDest &d, vb_frame_stats *stats) {
+    r->retries = 0;
+    for (uint32_t attempt = 0;; attempt++) {
+        int rc = frame_prepare(r, p, d);
+        if (rc == VB_OK) rc = frame_launch(r);
+        if (rc == VB_OK) rc = vb_frame_finish(r, stats);
+        if (rc == VB_E_BUMP_OVERFLOW) {
+            if (r->xc.enabled) {
+                // every attempt of an exchanged frame is a collective step (all GPUs advance their epoch together): grow what
+                // overflowed here and let the caller re-issue the frame on every GPU
+                grow_arenas(r);
+                r->err = "bump overflow in an exchanged frame: re-issue the frame on every GPU";
+            } else if (attempt >= r->max_retries) {
+                r->err = "bump overflow persisted";
+            } else {
+                grow_arenas(r);
+                r->retries++;
+                continue;
+            }
+        }
+        // a re-run after an arena overflow simply copies again
+        return d.host_out ? wait_copies(r, rc) : rc;
+    }
 }
 
 extern "C" int vb_render_resident(vb_renderer *r, const vb_params *p, void *out_device, vb_frame_stats *stats) {
     if (!r || !p) return VB_E_INVALID;
-    {
-        int rcd = drain_stream(r);
-        if (rcd) return rcd;
-    }
-    if (!r->have_scene) return VB_E_NO_SCENE;
-    r->retries = 0;
-    for (uint32_t attempt = 0;; attempt++) {
-        int rc = vb_render_enqueue(r, p, out_device);
-        if (rc) return rc;
-        CK(cudaStreamSynchronize(r->stream));
-        r->frame_pending = false;
-        if (r->h_bump->failed == 0) break;
-        if (r->xc.enabled) {
-            // every attempt of an exchanged frame is a collective step (all GPUs advance their epoch together): grow what
-            // overflowed here and let the caller re-issue the frame on every GPU
-            grow_arenas(r);
-            fill_stats(r, stats);
-            r->err = "bump overflow in an exchanged frame: re-issue the frame on every GPU";
-            return VB_E_BUMP_OVERFLOW;
-        }
-        if (attempt >= r->max_retries) {
-            fill_stats(r, stats);
-            r->err = "bump overflow persisted";
-            return VB_E_BUMP_OVERFLOW;
-        }
-        grow_arenas(r);
-        r->retries++;
-    }
-    fill_stats(r, stats);
-    return VB_OK;
+    int rc = drain_stream(r);
+    if (rc) return rc;
+    return render_attempts(r, p, FrameDest{out_device, nullptr, 1u, 0u, false}, stats);
 }
 
 extern "C" int vb_render_uploaded(vb_renderer *r, const vb_params *p, void *out, uint32_t out_is_device, vb_frame_stats *stats) {
     if (!r || !p || !out) return VB_E_INVALID;
-    r->host_out = out_is_device ? nullptr : out;
-    int rc = vb_render_resident(r, p, out_is_device ? out : nullptr, stats);
-    r->host_out = nullptr;
-    if (!out_is_device) {
-        // the band copies were queued behind the fine bands; a re-run after an arena overflow simply copies again
-        cudaError_t e = cudaStreamSynchronize(r->copy_stream);
-        if (rc == VB_OK && e != cudaSuccess) {
-            r->err = std::string("copy stream: ") + cudaGetErrorString(e);
-            return VB_E_CUDA;
-        }
-    }
-    return rc;
+    int rc = drain_stream(r);
+    if (rc) return rc;
+    const FrameDest d{out_is_device ? out : nullptr, out_is_device ? nullptr : out, r->readback_bands, 0u, false};
+    return render_attempts(r, p, d, stats);
 }
 
 extern "C" int vb_render(vb_renderer *r, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
@@ -1009,163 +851,19 @@ extern "C" int vb_render(vb_renderer *r, const uint8_t *scene, size_t scene_len,
     return vb_render_uploaded(r, p, out, out_is_device, stats);
 }
 
-// ---- streaming: vb_render_begin / vb_readback_wait ------------------------------------------------------------------------
-// Back-to-back frames with HOST buffers (a viewer / exporter reading every frame back, examples/headless/src/main.rs:188-210).
-// Three frames are in flight: vb_render_begin(k) uploads frame k's scene into the free scene slot on the upload stream and
-// enqueues its rasterisation and read-back; it then makes sure frame k-1 was RASTERISED without an arena overflow and that
-// frame k-2's PIXELS are on the host. In steady state the GPU sees  upload(k+1) | raster(k) | read-back(k-1)  side by side and a
-// frame costs max(raster, read-back) instead of their sum. On return every frame before the previous one is complete in its
-// out_host and `stats` describes frame k-2 (zeros while there is none); vb_readback_wait completes the rest. THREE alternating
-// out_host buffers are needed. An arena overflow is found at the rasterisation check; that frame (and the one enqueued behind
-// it) is then re-run synchronously with grown arenas -- rare (first frames of a new scene size) and exact.
-static int rerun_frame_sync(vb_renderer *r, uint32_t q, vb_frame_stats *stats) {
-    const uint32_t slot = r->ring[q].slot;
-    select_slot(r, slot);
-    r->host_out = r->ring[q].out_host;
-    r->use_alt = slot != 0u;
-    const uint32_t bands = r->readback_bands;
-    r->readback_bands = 1;
-    int rc = vb_render_resident(r, &r->ring[q].params, nullptr, stats);
-    r->readback_bands = bands;
-    r->host_out = nullptr;
-    r->use_alt = false;
-    cudaError_t e = cudaStreamSynchronize(r->copy_stream);
-    if (rc == VB_OK && e != cudaSuccess) {
-        r->err = std::string("copy stream: ") + cudaGetErrorString(e);
-        rc = VB_E_CUDA;
-    }
-    return rc;
-}
-
-// Frame in ring entry q: wait for its kernels, look at its bump counters, re-run on overflow (together with the younger frame
-// enqueued behind it, ring entry `younger`, or -1).
-static int check_raster(vb_renderer *r, uint32_t q, int younger) {
-    vb_renderer::RingFrame &f = r->ring[q];
-    if (!f.pending || f.raster_checked) return VB_OK;
-    const uint32_t keep = r->cur_slot;
-    CK(cudaEventSynchronize(r->raster_done[f.slot]));
-    select_slot(r, f.slot);
-    int rc = VB_OK;
-    if (r->h_bump->failed != 0u) {
-        CK(cudaStreamSynchronize(r->stream));
-        CK(cudaStreamSynchronize(r->copy_stream));
-        grow_arenas(r);
-        rc = rerun_frame_sync(r, q, &f.stats);
-        CK(cudaEventRecord(r->copy_done[q], r->copy_stream));
-        if (rc == VB_OK && younger >= 0 && r->ring[younger].pending) {
-            select_slot(r, r->ring[younger].slot);
-            if (r->h_bump->failed != 0u) {
-                rc = rerun_frame_sync(r, (uint32_t)younger, &r->ring[younger].stats);
-                CK(cudaEventRecord(r->raster_done[r->ring[younger].slot], r->stream));
-                CK(cudaEventRecord(r->copy_done[younger], r->copy_stream));
-            }
-        }
-    } else {
-        r->retries = 0;
-        fill_stats(r, &f.stats);
-    }
-    f.raster_checked = true;
-    select_slot(r, keep);
-    return rc;
-}
-
-static int complete_host(vb_renderer *r, uint32_t q, vb_frame_stats *stats) {
-    vb_renderer::RingFrame &f = r->ring[q];
-    if (!f.pending) return VB_OK;
-    int rc = check_raster(r, q, -1);
-    CK(cudaEventSynchronize(r->copy_done[q]));
-    if (stats) *stats = f.stats;
-    f.pending = false;
-    return rc;
-}
-
-extern "C" int vb_render_begin(vb_renderer *r, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
-                               uint32_t ramp_w, uint32_t ramp_h, const uint8_t *atlas, uint32_t atlas_w, uint32_t atlas_h,
-                               const vb_params *p, void *out_host, vb_frame_stats *stats) {
-    if (!r || !p || !out_host) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    if (stats) memset(stats, 0, sizeof *stats);
-    struct Guard {
-        vb_renderer *r;
-        ~Guard() { r->in_stream_call = false; }
-    } guard{r};
-    r->in_stream_call = true;
-    const uint64_t k = r->stream_seq;
-    const uint32_t slot = (uint32_t)(k & 1u), q = (uint32_t)(k % 3u), q1 = (uint32_t)((k + 2u) % 3u), q2 = (uint32_t)((k + 1u) % 3u);
-    // frame k-2 (same scene slot, same device target) was checked by the previous call; frame k-3 (ring entry q) is complete
-    select_slot(r, slot);
-    int rc = upload_on(r, r->upload_stream, scene, scene_len, layout, ramps, ramp_w, ramp_h, atlas, atlas_w, atlas_h);
-    if (rc) return rc;
-    CK(cudaEventRecord(r->upload_done[slot], r->upload_stream));
-    CK(cudaStreamWaitEvent(r->stream, r->upload_done[slot], 0));
-    if (k >= 2u && r->ring[q2].pending) CK(cudaStreamWaitEvent(r->stream, r->copy_done[q2], 0)); // its read-back still reads this target
-    const uint32_t bands = r->readback_bands;
-    r->readback_bands = 1; // the whole read-back overlaps the next frames: no reason to split fine
-    r->host_out = out_host;
-    r->use_alt = slot != 0u;
-    rc = vb_render_enqueue(r, p, nullptr);
-    r->host_out = nullptr;
-    r->use_alt = false;
-    r->readback_bands = bands;
-    if (rc) return rc;
-    r->frame_pending = false;
-    CK(cudaEventRecord(r->raster_done[slot], r->stream));
-    CK(cudaEventRecord(r->copy_done[q], r->copy_stream));
-    r->ring[q].pending = true;
-    r->ring[q].raster_checked = false;
-    r->ring[q].params = *p;
-    r->ring[q].out_host = out_host;
-    r->ring[q].slot = slot;
-    memset(&r->ring[q].stats, 0, sizeof(vb_frame_stats));
-    r->stream_seq = k + 1u;
-    r->stream_pending = true;
-    // frame k-1: rasterised without overflow?  frame k-2: pixels on the host?
-    if (k >= 1u) rc = check_raster(r, q1, (int)q);
-    if (k >= 2u) {
-        const int rc2 = complete_host(r, q2, stats);
-        if (rc == VB_OK) rc = rc2;
-    }
-    return rc;
-}
-
-extern "C" int vb_readback_wait(vb_renderer *r) {
-    if (!r) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    struct Guard {
-        vb_renderer *r;
-        ~Guard() { r->in_stream_call = false; }
-    } guard{r};
-    r->in_stream_call = true;
-    int rc = VB_OK;
-    const uint64_t k = r->stream_seq; // the next frame number: complete k-3 .. k-1 in order
-    for (uint64_t j = k >= 3u ? k - 3u : 0u; j < k; j++) {
-        const uint32_t q = (uint32_t)(j % 3u);
-        const int younger = j + 1u < k ? (int)((j + 1u) % 3u) : -1;
-        int rc1 = check_raster(r, q, younger);
-        if (rc1 == VB_OK) rc1 = complete_host(r, q, nullptr);
-        if (rc == VB_OK) rc = rc1;
-    }
-    CK(cudaStreamSynchronize(r->copy_stream));
-    r->stream_pending = false;
-    return rc;
-}
-
 extern "C" int vb_run_stages(vb_renderer *r, const vb_params *p, int first, int last, void *out_device) {
     if (!r || !p || first < 0 || last >= VB_N_STAGE_IDS || first > last) return VB_E_INVALID;
-    if (!r->have_scene) return VB_E_NO_SCENE;
-    CK(cudaSetDevice(r->device));
+    if (!r->cur().have_scene) return VB_E_NO_SCENE;
+    CK(r->err, cudaSetDevice(r->device));
     int rc = prepare(r, p);
     if (rc) return rc;
-    void *out = nullptr;
+    FrameDest d{nullptr, nullptr, 1u, 0u, true};
     if (last == VB_STAGE_ID_FINE) {
-        if ((rc = pick_out(r, out_device, &out))) return rc;
-        r->out_dev = out;
+        d.out_dev = out_device;
+        if ((rc = pick_out(r, d))) return rc;
     }
-    r->zero_fine_queue = true;
-    rc = enqueue(r, first, last, out);
-    r->zero_fine_queue = false;
-    if (rc) return rc;
-    CK(cudaStreamSynchronize(r->stream));
+    if ((rc = enqueue(r, first, last, d))) return rc;
+    CK(r->err, cudaStreamSynchronize(r->stream));
     return VB_OK;
 }
 
@@ -1176,8 +874,8 @@ struct NamedBuf {
 };
 static std::vector<NamedBuf> named(vb_renderer *r) {
     const VbConfig &c = r->cfg;
-    const VbLayout &L = r->layout;
-    const VbBump &b = *r->h_bump;
+    const VbLayout &L = r->cur().layout;
+    const VbBump &b = *r->cur().h_bump;
     auto mn = [](uint64_t a, uint64_t b2) { return a < b2 ? a : b2; };
     const uint32_t wb = (c.width_in_tiles + 15u) / 16u, hb = (c.height_in_tiles + 15u) / 16u;
     const uint32_t aligned_n_bins = (wb * hb + 255u) & ~255u;
@@ -1203,24 +901,25 @@ static std::vector<NamedBuf> named(vb_renderer *r) {
 
 extern "C" int vb_debug_download(vb_renderer *r, const char *name, void *dst, size_t cap, size_t *bytes) {
     if (!r || !name) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
     if (!strcmp(name, "bump")) {
         if (bytes) *bytes = sizeof(VbBump);
-        if (dst && cap >= sizeof(VbBump)) CK(cudaMemcpy(dst, r->ctl.p, sizeof(VbBump), cudaMemcpyDeviceToHost));
+        if (dst && cap >= sizeof(VbBump)) CK(r->err, cudaMemcpy(dst, r->ctl.p, sizeof(VbBump), cudaMemcpyDeviceToHost));
         return VB_OK;
     }
     if (!strcmp(name, "seg_holes")) { // reserved-but-unused segment slots of the last frame (k_coarse.cu)
         if (bytes) *bytes = 4;
-        if (dst && cap >= 4) CK(cudaMemcpy(dst, (const uint32_t *)r->ctl.p + VB_CTL_SEG_HOLES, 4, cudaMemcpyDeviceToHost));
+        if (dst && cap >= 4) CK(r->err, cudaMemcpy(dst, (const uint32_t *)r->ctl.p + VB_CTL_SEG_HOLES, 4, cudaMemcpyDeviceToHost));
         return VB_OK;
     }
     if (!strcmp(name, "scene") || !strcmp(name, "ramps") || !strcmp(name, "atlas")) { // the uploaded / device-resolved inputs
-        const DevBuf &b = name[0] == 's' ? r->scene : (name[0] == 'r' ? r->ramps : r->atlas);
-        const size_t n = name[0] == 's' ? r->scene_words * 4 : (name[0] == 'r' ? (size_t)r->n_ramps * 512 * 4 : (size_t)r->atlas_w * r->atlas_h * 4);
+        const SceneSlot &s = r->cur();
+        const DevBuf &b = name[0] == 's' ? s.scene : (name[0] == 'r' ? s.ramps : s.atlas);
+        const size_t n = name[0] == 's' ? s.scene_words * 4 : (name[0] == 'r' ? (size_t)s.n_ramps * 512 * 4 : (size_t)s.atlas_w * s.atlas_h * 4);
         if (bytes) *bytes = n;
         const size_t c = n < cap ? n : cap;
-        if (dst && c) CK(cudaMemcpy(dst, b.p, c, cudaMemcpyDeviceToHost));
+        if (dst && c) CK(r->err, cudaMemcpy(dst, b.p, c, cudaMemcpyDeviceToHost));
         return VB_OK;
     }
     if (!strcmp(name, "config")) {
@@ -1232,7 +931,7 @@ extern "C" int vb_debug_download(vb_renderer *r, const char *name, void *dst, si
         if (!strcmp(name, nb.name)) {
             if (bytes) *bytes = nb.bytes;
             size_t n = nb.bytes < cap ? nb.bytes : cap;
-            if (dst && n) CK(cudaMemcpy(dst, nb.buf->p, n, cudaMemcpyDeviceToHost));
+            if (dst && n) CK(r->err, cudaMemcpy(dst, nb.buf->p, n, cudaMemcpyDeviceToHost));
             return VB_OK;
         }
     return VB_E_UNKNOWN_BUFFER;
@@ -1264,16 +963,16 @@ extern "C" int vb_set_occlusion_cull(vb_renderer *r, int on) {
 
 extern "C" int vb_debug_fine_traffic(vb_renderer *r, uint64_t *ptcl_words, uint64_t *segment_refs, uint64_t *fill_cmds) {
     if (!r) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
     unsigned long long *d = nullptr, h[3] = {0, 0, 0};
-    CK(cudaMalloc(&d, sizeof h));
-    CK(cudaMemset(d, 0, sizeof h));
+    CK(r->err, cudaMalloc(&d, sizeof h));
+    CK(r->err, cudaMemset(d, 0, sizeof h));
     uint32_t n = r->cfg.width_in_tiles * (r->cfg.win_ty1 - r->cfg.win_ty0);
     if (n) k_ptcl_stats<<<(n + 127) / 128, 128, 0, r->stream>>>(r->cfg, (const uint32_t *)r->ptcl.p,
                                                                 r->occlusion_cull ? (const uint32_t *)r->tile_start.p : nullptr, d);
-    CK(cudaStreamSynchronize(r->stream));
-    CK(cudaMemcpy(h, d, sizeof h, cudaMemcpyDeviceToHost));
+    CK(r->err, cudaStreamSynchronize(r->stream));
+    CK(r->err, cudaMemcpy(h, d, sizeof h, cudaMemcpyDeviceToHost));
     cudaFree(d);
     if (ptcl_words) *ptcl_words = h[0];
     if (segment_refs) *segment_refs = h[1];
@@ -1283,8 +982,8 @@ extern "C" int vb_debug_fine_traffic(vb_renderer *r, uint64_t *ptcl_words, uint6
 
 extern "C" int vb_debug_upload(vb_renderer *r, const char *name, const void *src, size_t bytes) {
     if (!r || !name || !src) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
     if (!strcmp(name, "lines")) {
         uint32_t n = (uint32_t)(bytes / sizeof(VbLineSoup));
         if (n > r->cap_lines) {
@@ -1292,15 +991,15 @@ extern "C" int vb_debug_upload(vb_renderer *r, const char *name, const void *src
             int rc = ensure(r, r->lines, (size_t)r->cap_lines * sizeof(VbLineSoup));
             if (rc) return rc;
         }
-        CK(cudaMemcpy(r->lines.p, src, (size_t)n * sizeof(VbLineSoup), cudaMemcpyHostToDevice));
+        CK(r->err, cudaMemcpy(r->lines.p, src, (size_t)n * sizeof(VbLineSoup), cudaMemcpyHostToDevice));
         VbBump *bump = (VbBump *)r->ctl.p;
-        CK(cudaMemcpy(&bump->lines, &n, 4, cudaMemcpyHostToDevice));
-        r->h_bump->lines = n;
+        CK(r->err, cudaMemcpy(&bump->lines, &n, 4, cudaMemcpyHostToDevice));
+        r->cur().h_bump->lines = n;
         return VB_OK;
     }
     if (!strcmp(name, "path_bboxes")) {
         if (bytes > r->path_bboxes.cap) return VB_E_INVALID;
-        CK(cudaMemcpy(r->path_bboxes.p, src, bytes, cudaMemcpyHostToDevice));
+        CK(r->err, cudaMemcpy(r->path_bboxes.p, src, bytes, cudaMemcpyHostToDevice));
         return VB_OK;
     }
     return VB_E_UNKNOWN_BUFFER;
@@ -1321,377 +1020,40 @@ extern "C" float vb_last_frame_ms(vb_renderer *r) {
 // ---- CUDA IPC helpers (one process per GPU: the frame buffer of rank 0 mapped into the other ranks) ----------------------
 extern "C" int vb_frame_alloc(vb_renderer *r, size_t bytes, void **device_ptr) {
     if (!r || !device_ptr || !bytes) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaMalloc(device_ptr, bytes));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaMalloc(device_ptr, bytes));
     return VB_OK;
 }
 extern "C" int vb_frame_free(vb_renderer *r, void *device_ptr) {
     if (!r) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
-    if (device_ptr) CK(cudaFree(device_ptr));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
+    if (device_ptr) CK(r->err, cudaFree(device_ptr));
     return VB_OK;
 }
 extern "C" int vb_ipc_export(vb_renderer *r, void *device_ptr, uint8_t handle[64]) {
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
     if (!r || !device_ptr || !handle) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
+    CK(r->err, cudaSetDevice(r->device));
     cudaIpcMemHandle_t h;
-    CK(cudaIpcGetMemHandle(&h, device_ptr));
+    CK(r->err, cudaIpcGetMemHandle(&h, device_ptr));
     memcpy(handle, &h, 64);
     return VB_OK;
 }
 extern "C" int vb_ipc_open(vb_renderer *r, const uint8_t handle[64], void **device_ptr) {
     if (!r || !handle || !device_ptr) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
+    CK(r->err, cudaSetDevice(r->device));
     cudaIpcMemHandle_t h;
     memcpy(&h, handle, 64);
-    CK(cudaIpcOpenMemHandle(device_ptr, h, cudaIpcMemLazyEnablePeerAccess));
+    CK(r->err, cudaIpcOpenMemHandle(device_ptr, h, cudaIpcMemLazyEnablePeerAccess));
     return VB_OK;
 }
 extern "C" int vb_ipc_close(vb_renderer *r, void *device_ptr) {
     if (!r || !device_ptr) return VB_E_INVALID;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
-    CK(cudaIpcCloseMemHandle(device_ptr));
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
+    CK(r->err, cudaIpcCloseMemHandle(device_ptr));
     return VB_OK;
-}
-
-// ---- vb_group: one frame on several devices of one box, one host thread ---------------------------------------------------
-struct vb_group {
-    std::vector<vb_renderer *> subs;
-    std::vector<int> devices;
-    std::vector<uint32_t> bounds;   // tile-row boundaries, subs.size() + 1 entries
-    std::vector<float> ms;          // device time of the last frame per renderer
-    std::vector<char> peer_ok;      // renderer i can store into device 0's memory
-    std::vector<cudaEvent_t> done;  // per renderer: its stripe is in the frame
-    void *frame = nullptr;          // assembled frame on devices[0]
-    size_t frame_cap = 0;
-    uint32_t bounds_h = 0;          // height in tiles the boundaries were made for
-    bool balancing = true;
-    bool exchange = false;          // flatten sharded by tag range, lines exchanged through peer memory (k_exchange.cu)
-    bool shared_device = false;     // two renderers on one GPU (tests)
-    std::string err;
-};
-
-extern "C" int vb_group_new(const int32_t *devices, uint32_t n, const vb_options *opt, vb_group **out) {
-    if (!devices || !n || n > 64 || !out) return VB_E_INVALID;
-    vb_group *g = new vb_group();
-    for (uint32_t i = 0; i < n; i++) {
-        vb_options o{};
-        if (opt) o = *opt;
-        o.device = devices[i];
-        vb_renderer *r = nullptr;
-        int rc = vb_renderer_new(&o, &r);
-        if (rc) {
-            vb_group_free(g);
-            return rc;
-        }
-        g->subs.push_back(r);
-        g->devices.push_back(devices[i]);
-        cudaEvent_t ev = nullptr;
-        cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-        g->done.push_back(ev);
-        // stores of `fine` on device i land in device 0's frame buffer through peer mapping (NVLink / NVSwitch)
-        char ok = 1;
-        if (devices[i] != devices[0]) {
-            int can = 0;
-            cudaSetDevice(devices[i]);
-            if (cudaDeviceCanAccessPeer(&can, devices[i], devices[0]) != cudaSuccess || !can) ok = 0;
-            else {
-                cudaError_t e = cudaDeviceEnablePeerAccess(devices[0], 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) ok = 0;
-                cudaGetLastError();
-            }
-        }
-        g->peer_ok.push_back(ok);
-    }
-    g->ms.assign(n, 0.0f);
-    *out = g;
-    return VB_OK;
-}
-
-extern "C" void vb_group_free(vb_group *g) {
-    if (!g) return;
-    for (vb_renderer *r : g->subs) vb_renderer_free(r);
-    if (!g->devices.empty()) cudaSetDevice(g->devices[0]);
-    if (g->frame) cudaFree(g->frame);
-    for (cudaEvent_t ev : g->done)
-        if (ev) cudaEventDestroy(ev);
-    delete g;
-}
-extern "C" uint32_t vb_group_size(const vb_group *g) { return g ? (uint32_t)g->subs.size() : 0u; }
-extern "C" vb_renderer *vb_group_renderer(vb_group *g, uint32_t i) { return g && i < g->subs.size() ? g->subs[i] : nullptr; }
-extern "C" const char *vb_group_last_error(vb_group *g) { return g ? g->err.c_str() : ""; }
-extern "C" int vb_group_set_balancing(vb_group *g, int on) {
-    if (!g) return VB_E_INVALID;
-    g->balancing = on != 0;
-    return VB_OK;
-}
-extern "C" void *vb_group_frame(vb_group *g, size_t *bytes) {
-    if (!g) return nullptr;
-    if (bytes) *bytes = g->frame_cap;
-    return g->frame;
-}
-extern "C" int vb_group_stripes(vb_group *g, uint32_t *boundaries, float *device_ms) {
-    if (!g) return VB_E_INVALID;
-    if (boundaries)
-        for (size_t i = 0; i < g->bounds.size(); i++) boundaries[i] = g->bounds[i];
-    if (device_ms)
-        for (size_t i = 0; i < g->ms.size(); i++) device_ms[i] = g->ms[i];
-    return VB_OK;
-}
-
-// Move the stripe boundaries so that the device times of the last frame would have been equal, assuming the cost of a stripe is
-// spread evenly over its tile rows (piecewise-linear cumulative cost); damped, every stripe keeps at least one tile row.
-static void group_rebalance(vb_group *g, uint32_t ht) {
-    const size_t n = g->subs.size();
-    if (g->bounds.size() != n + 1 || g->bounds_h != ht) {
-        g->bounds.assign(n + 1, 0u);
-        for (size_t i = 0; i <= n; i++) g->bounds[i] = (uint32_t)((uint64_t)ht * i / n);
-        g->bounds_h = ht;
-        return;
-    }
-    if (!g->balancing || n < 2 || ht < n) return;
-    double total = 0.0, lo = 1e30, hi = 0.0;
-    for (size_t i = 0; i < n; i++) {
-        if (!(g->ms[i] > 0.0f)) return; // no measurement yet
-        total += g->ms[i];
-        lo = std::min<double>(lo, g->ms[i]);
-        hi = std::max<double>(hi, g->ms[i]);
-    }
-    if (hi - lo < 0.06 * (total / n)) return; // balanced within noise: keep the stripes (and the captured graphs)
-    std::vector<uint32_t> nb(n + 1, 0u);
-    nb[n] = ht;
-    size_t seg = 0;
-    double acc = 0.0; // cost of the stripes before `seg`
-    for (size_t k = 1; k < n; k++) {
-        const double want = total * k / n;
-        while (seg + 1 < n && acc + g->ms[seg] < want) acc += g->ms[seg++];
-        const double rows = (double)(g->bounds[seg + 1] - g->bounds[seg]);
-        const double frac = g->ms[seg] > 0.0f ? (want - acc) / g->ms[seg] : 0.0;
-        const double ideal = g->bounds[seg] + rows * frac;
-        const double damped = 0.5 * g->bounds[k] + 0.5 * ideal;
-        nb[k] = (uint32_t)(damped + 0.5);
-    }
-    for (size_t k = 1; k < n; k++) { // monotone, at least one row each
-        if (nb[k] < nb[k - 1] + 1u) nb[k] = nb[k - 1] + 1u;
-    }
-    for (size_t k = n - 1; k >= 1; k--) {
-        if (nb[k] > nb[k + 1] - 1u) nb[k] = nb[k + 1] - 1u;
-    }
-    g->bounds = nb;
-}
-
-#define GCK(call)                                                                                 \
-    do {                                                                                          \
-        cudaError_t e_ = (call);                                                                  \
-        if (e_ != cudaSuccess) {                                                                  \
-            g->err = std::string(#call) + ": " + cudaGetErrorString(e_);                          \
-            return VB_E_CUDA;                                                                     \
-        }                                                                                         \
-    } while (0)
-
-// (re)build the exchange arenas for the uploaded scene and introduce the renderers to each other
-static int group_setup_exchange(vb_group *g) {
-    const uint32_t n = (uint32_t)g->subs.size();
-    if (n > 8u) return VB_E_INVALID;
-    std::vector<void *> arenas(n, nullptr);
-    for (uint32_t i = 0; i < n; i++) {
-        int rc = vb_exchange_configure(g->subs[i], i, n, &arenas[i], nullptr);
-        if (rc) {
-            g->err = g->subs[i]->err;
-            return rc;
-        }
-    }
-    for (uint32_t i = 0; i < n; i++) {
-        for (uint32_t j = 0; j < n; j++) {
-            if (i == j) continue;
-            if (g->devices[i] != g->devices[j]) { // every GPU reads every other GPU's arena
-                int can = 0;
-                cudaSetDevice(g->devices[i]);
-                if (cudaDeviceCanAccessPeer(&can, g->devices[i], g->devices[j]) != cudaSuccess || !can) {
-                    g->err = "exchange needs peer access between all devices of the group";
-                    return VB_E_CUDA;
-                }
-                cudaError_t e = cudaDeviceEnablePeerAccess(g->devices[j], 0);
-                if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) {
-                    g->err = std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(e);
-                    return VB_E_CUDA;
-                }
-                cudaGetLastError();
-            }
-            int rc = vb_exchange_attach(g->subs[i], j, arenas[j]);
-            if (rc) return rc;
-        }
-    }
-    bool shared_device = false;
-    for (uint32_t i = 0; i < n; i++)
-        for (uint32_t j = i + 1; j < n; j++) shared_device = shared_device || g->devices[i] == g->devices[j];
-    g->shared_device = shared_device;
-    for (uint32_t i = 0; i < n; i++) {
-        int rc = vb_exchange_enable(g->subs[i], 1);
-        if (rc) return rc;
-        // renderers that share a GPU (tests): no graph (re-)instantiation while a peer's wait kernel is resident on that GPU
-        if (shared_device) g->subs[i]->use_graph = false;
-    }
-    return VB_OK;
-}
-
-extern "C" int vb_group_set_exchange(vb_group *g, int on) {
-    if (!g) return VB_E_INVALID;
-    g->exchange = on != 0;
-    if (!g->exchange) {
-        for (vb_renderer *r : g->subs) vb_exchange_enable(r, 0);
-        return VB_OK;
-    }
-    for (vb_renderer *r : g->subs)
-        if (!r->have_scene) return VB_OK; // arenas are built by the next vb_group_scene_upload
-    return group_setup_exchange(g);
-}
-
-extern "C" int vb_group_scene_upload(vb_group *g, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
-                                     uint32_t ramp_w, uint32_t ramp_h, const uint8_t *atlas, uint32_t atlas_w, uint32_t atlas_h) {
-    if (!g) return VB_E_INVALID;
-    // every device pulls the scene over its own PCIe link (asynchronous per renderer, so the copies run side by side)
-    for (vb_renderer *r : g->subs) {
-        int rc = vb_scene_upload(r, scene, scene_len, layout, ramps, ramp_w, ramp_h, atlas, atlas_w, atlas_h);
-        if (rc) {
-            g->err = r->err;
-            return rc;
-        }
-    }
-    return g->exchange ? group_setup_exchange(g) : VB_OK;
-}
-
-// out: nullptr (group frame), a device pointer on devices[0], or (host_out) a host pointer
-static int group_render(vb_group *g, const vb_params *p, void *out_device, void *host_out, vb_frame_stats *stats) {
-    if (!g || !p || p->bin_row1 > p->bin_row0 || p->tile_row1 > p->tile_row0) return VB_E_INVALID;
-    const size_t n = g->subs.size();
-    const uint32_t ht = (p->height + 15u) / 16u;
-    if (g->exchange && ht < n) {
-        g->err = "exchange needs at least one tile row per device";
-        return VB_E_INVALID;
-    }
-    group_rebalance(g, ht);
-    const size_t pitch = (size_t)p->width * 4u;
-    void *frame = out_device;
-    if (!host_out && !frame) {
-        const size_t need = pitch * p->height;
-        if (g->frame_cap < need) {
-            GCK(cudaSetDevice(g->devices[0]));
-            if (g->frame) GCK(cudaFree(g->frame));
-            g->frame = nullptr;
-            g->frame_cap = 0;
-            GCK(cudaMalloc(&g->frame, need));
-            g->frame_cap = need;
-        }
-        frame = g->frame;
-    }
-    // enqueue every device's stripe, then complete them (one host thread; the devices run side by side)
-    std::vector<vb_params> ps(n, *p);
-    int result = VB_OK;
-    for (uint32_t attempt = 0;; attempt++) {
-        if (g->exchange)
-            for (vb_renderer *r : g->subs) vb_exchange_set_bounds(r, g->bounds.data());
-        const bool halves = g->exchange && g->shared_device;
-        // phases: 0 = configs and arenas of every renderer, 1 (and 2) = the launches, last = the read-backs of a host
-        // destination. A copy into pageable host memory blocks the host until it is done, so it must not be issued before
-        // every renderer's frame has been launched (with the exchange on, a frame waits for its peers).
-        const int n_launch = halves ? 2 : 1;
-        const bool late_copy = host_out != nullptr && g->exchange; // without the exchange every frame queues its own read-back
-        for (int phase = 0; phase < 1 + n_launch + (late_copy ? 1 : 0); phase++) {
-            for (size_t i = 0; i < n; i++) {
-                vb_renderer *r = g->subs[i];
-                ps[i].tile_row0 = g->bounds[i];
-                ps[i].tile_row1 = g->bounds[i + 1];
-                if (ps[i].tile_row1 <= ps[i].tile_row0) continue; // more devices than tile rows (never with the exchange on)
-                const size_t row0 = (size_t)g->bounds[i] * 16u;
-                // device destination: straight into the frame on devices[0] when peer-mapped; otherwise (and for a host
-                // destination) the renderer's own target
-                void *dst = (!host_out && g->peer_ok[i]) ? (char *)frame + row0 * pitch : nullptr;
-                if (host_out && !late_copy) { // the frame copies its stripe to the host itself, on the renderer's copy stream
-                    r->host_out = (char *)host_out + row0 * pitch;
-                    r->readback_bands = 1;
-                }
-                int rc = VB_OK;
-                if (phase == 0) rc = frame_prepare(r, &ps[i], dst);
-                else if (phase <= n_launch) rc = halves ? frame_launch_half(r, phase - 1) : frame_launch(r);
-                else {
-                    const size_t h1 = std::min<size_t>((size_t)g->bounds[i + 1] * 16u, p->height);
-                    cudaSetDevice(r->device);
-                    if (h1 > row0 && cudaMemcpyAsync((char *)host_out + row0 * pitch, r->out_dev, (h1 - row0) * pitch, cudaMemcpyDeviceToHost, r->stream) != cudaSuccess)
-                        rc = VB_E_CUDA;
-                }
-                if (rc) {
-                    for (vb_renderer *q : g->subs) q->host_out = nullptr;
-                    g->err = r->err;
-                    return rc;
-                }
-            }
-        }
-        result = VB_OK;
-        bool redo = false;
-        for (size_t i = 0; i < n; i++) {
-            vb_renderer *r = g->subs[i];
-            if (ps[i].tile_row1 <= ps[i].tile_row0) {
-                if (stats) memset(&stats[i], 0, sizeof(vb_frame_stats));
-                continue;
-            }
-            const size_t row0 = (size_t)g->bounds[i] * 16u;
-            void *dst = (!host_out && g->peer_ok[i]) ? (char *)frame + row0 * pitch : nullptr;
-            int rc = vb_frame_finish(r, stats ? &stats[i] : nullptr);
-            if (rc == VB_E_BUMP_OVERFLOW) {
-                if (g->exchange) { // an exchanged frame is re-issued on EVERY device (epochs advance together)
-                    grow_arenas(r);
-                    redo = true;
-                    rc = VB_OK;
-                } else {
-                    // grow and re-run (first frames); with a host destination the re-run queues its read-back again
-                    rc = vb_render_resident(r, &ps[i], dst, stats ? &stats[i] : nullptr);
-                }
-            }
-            g->ms[i] = vb_last_frame_ms(r);
-            if (rc == VB_OK && host_out && !late_copy) {
-                cudaSetDevice(r->device);
-                if (cudaStreamSynchronize(r->copy_stream) != cudaSuccess) rc = VB_E_CUDA;
-            }
-            r->host_out = nullptr;
-            if (rc == VB_OK && !host_out && !g->peer_ok[i]) {
-                // no peer mapping between these two devices: stage through the renderer's own target
-                const size_t h0 = row0, h1 = std::min<size_t>((size_t)g->bounds[i + 1] * 16u, p->height);
-                cudaSetDevice(r->device);
-                if (h1 > h0 && (cudaMemcpyPeerAsync((char *)frame + row0 * pitch, g->devices[0], r->out_dev, r->device, (h1 - h0) * pitch, r->stream) != cudaSuccess ||
-                                cudaStreamSynchronize(r->stream) != cudaSuccess))
-                    rc = VB_E_CUDA;
-            }
-            if (rc && result == VB_OK) {
-                result = rc;
-                g->err = r->err;
-            }
-        }
-        if (!redo || result != VB_OK) break;
-        if (attempt >= 8u) {
-            g->err = "bump overflow persisted in an exchanged frame; failed bits per renderer:";
-            for (vb_renderer *q : g->subs) g->err += " 0x" + std::to_string(q->h_bump->failed);
-            return VB_E_BUMP_OVERFLOW;
-        }
-    }
-    return result;
-}
-
-extern "C" int vb_group_render_resident(vb_group *g, const vb_params *p, void *out_device, vb_frame_stats *stats) {
-    return group_render(g, p, out_device, nullptr, stats);
-}
-
-extern "C" int vb_group_render(vb_group *g, const uint8_t *scene, size_t scene_len, const vb_layout *layout, const uint32_t *ramps,
-                               uint32_t ramp_w, uint32_t ramp_h, const uint8_t *atlas, uint32_t atlas_w, uint32_t atlas_h, const vb_params *p,
-                               void *out, uint32_t out_is_device, vb_frame_stats *stats) {
-    if (!g || !p) return VB_E_INVALID;
-    int rc = vb_group_scene_upload(g, scene, scene_len, layout, ramps, ramp_w, ramp_h, atlas, atlas_w, atlas_h);
-    if (rc) return rc;
-    if (out && !out_is_device) return group_render(g, p, nullptr, out, stats);
-    return group_render(g, p, out, nullptr, stats);
 }
 
 
@@ -1704,8 +1066,9 @@ extern "C" int vb_scene_upload_streams(vb_renderer *r, const vb_encoding_streams
         return VB_E_INVALID;
     int rc = drain_stream(r);
     if (rc) return rc;
-    CK(cudaSetDevice(r->device));
+    CK(r->err, cudaSetDevice(r->device));
     cudaStream_t st = r->stream;
+    SceneSlot &sl = r->cur();
     struct Patch { uint32_t word, value; };
     struct Ramp { uint32_t first_stop, n_stops, premul, pad; };
     std::vector<Patch> patches;
@@ -1775,66 +1138,67 @@ extern "C" int vb_scene_upload_streams(vb_renderer *r, const vb_encoding_streams
     const uint32_t atlas_h = (y + shelf_h) > 1u ? (y + shelf_h) : 1u;
 
     // the six streams go straight to their places in the packed buffer
-    if ((rc = ensure(r, r->scene, total_words * 4 + 64))) return rc;
-    char *base = (char *)r->scene.p;
-    if (e->n_path_tags) CK(cudaMemcpyAsync(base, e->path_tags, e->n_path_tags, cudaMemcpyHostToDevice, st));
-    if (e->n_path_data) CK(cudaMemcpyAsync(base + (size_t)L.path_data_base * 4, e->path_data, (size_t)e->n_path_data * 4, cudaMemcpyHostToDevice, st));
-    if (e->n_draw_tags) CK(cudaMemcpyAsync(base + (size_t)L.draw_tag_base * 4, e->draw_tags, (size_t)e->n_draw_tags * 4, cudaMemcpyHostToDevice, st));
-    if (e->n_draw_data) CK(cudaMemcpyAsync(base + (size_t)L.draw_data_base * 4, e->draw_data, (size_t)e->n_draw_data * 4, cudaMemcpyHostToDevice, st));
-    if (e->n_transforms) CK(cudaMemcpyAsync(base + (size_t)L.transform_base * 4, e->transforms, (size_t)e->n_transforms * 24, cudaMemcpyHostToDevice, st));
-    if (e->n_styles) CK(cudaMemcpyAsync(base + (size_t)L.style_base * 4, e->styles, (size_t)e->n_styles * 8, cudaMemcpyHostToDevice, st));
+    if ((rc = ensure(r, sl.scene, total_words * 4 + 64))) return rc;
+    char *base = (char *)sl.scene.p;
+    if (e->n_path_tags) CK(r->err, cudaMemcpyAsync(base, e->path_tags, e->n_path_tags, cudaMemcpyHostToDevice, st));
+    if (e->n_path_data) CK(r->err, cudaMemcpyAsync(base + (size_t)L.path_data_base * 4, e->path_data, (size_t)e->n_path_data * 4, cudaMemcpyHostToDevice, st));
+    if (e->n_draw_tags) CK(r->err, cudaMemcpyAsync(base + (size_t)L.draw_tag_base * 4, e->draw_tags, (size_t)e->n_draw_tags * 4, cudaMemcpyHostToDevice, st));
+    if (e->n_draw_data) CK(r->err, cudaMemcpyAsync(base + (size_t)L.draw_data_base * 4, e->draw_data, (size_t)e->n_draw_data * 4, cudaMemcpyHostToDevice, st));
+    if (e->n_transforms) CK(r->err, cudaMemcpyAsync(base + (size_t)L.transform_base * 4, e->transforms, (size_t)e->n_transforms * 24, cudaMemcpyHostToDevice, st));
+    if (e->n_styles) CK(r->err, cudaMemcpyAsync(base + (size_t)L.style_base * 4, e->styles, (size_t)e->n_styles * 8, cudaMemcpyHostToDevice, st));
     // patches, ramp descriptors and stops in one staging buffer
     const size_t pb = patches.size() * sizeof(Patch), rb = ramps.size() * sizeof(Ramp), sb = stops.size() * sizeof(vb_ramp_stop);
     const size_t o_r = (pb + 15) & ~(size_t)15, o_s = (o_r + rb + 15) & ~(size_t)15;
     if ((rc = ensure(r, r->resolve_tmp, o_s + sb + 16))) return rc;
     char *tmp = (char *)r->resolve_tmp.p;
-    if (pb) CK(cudaMemcpyAsync(tmp, patches.data(), pb, cudaMemcpyHostToDevice, st));
-    if (rb) CK(cudaMemcpyAsync(tmp + o_r, ramps.data(), rb, cudaMemcpyHostToDevice, st));
-    if (sb) CK(cudaMemcpyAsync(tmp + o_s, stops.data(), sb, cudaMemcpyHostToDevice, st));
-    vb_launch_resolve_finish((uint32_t *)r->scene.p, e->n_path_tags, e->n_open_clips, padded, L.draw_tag_base + e->n_draw_tags, tmp,
+    if (pb) CK(r->err, cudaMemcpyAsync(tmp, patches.data(), pb, cudaMemcpyHostToDevice, st));
+    if (rb) CK(r->err, cudaMemcpyAsync(tmp + o_r, ramps.data(), rb, cudaMemcpyHostToDevice, st));
+    if (sb) CK(r->err, cudaMemcpyAsync(tmp + o_s, stops.data(), sb, cudaMemcpyHostToDevice, st));
+    vb_launch_resolve_finish((uint32_t *)sl.scene.p, e->n_path_tags, e->n_open_clips, padded, L.draw_tag_base + e->n_draw_tags, tmp,
                              (uint32_t)patches.size(), st);
-    r->n_ramps = (uint32_t)ramps.size();
-    if ((rc = ensure(r, r->ramps, (size_t)r->n_ramps * 512 * 4))) return rc;
-    vb_launch_make_ramps(tmp + o_r, tmp + o_s, r->n_ramps, (uint32_t *)r->ramps.p, st);
-    r->atlas_w = atlas_w;
-    r->atlas_h = atlas_h;
-    if ((rc = ensure(r, r->atlas, (size_t)atlas_w * atlas_h * 4))) return rc;
-    CK(cudaMemsetAsync(r->atlas.p, 0, (size_t)atlas_w * atlas_h * 4, st));
+    sl.n_ramps = (uint32_t)ramps.size();
+    if ((rc = ensure(r, sl.ramps, (size_t)sl.n_ramps * 512 * 4))) return rc;
+    vb_launch_make_ramps(tmp + o_r, tmp + o_s, sl.n_ramps, (uint32_t *)sl.ramps.p, st);
+    sl.atlas_w = atlas_w;
+    sl.atlas_h = atlas_h;
+    if ((rc = ensure(r, sl.atlas, (size_t)atlas_w * atlas_h * 4))) return rc;
+    CK(r->err, cudaMemsetAsync(sl.atlas.p, 0, (size_t)atlas_w * atlas_h * 4, st));
     for (const Placed &q : placed)
         if (q.key && q.w && q.h)
-            CK(cudaMemcpy2DAsync((char *)r->atlas.p + ((size_t)q.y * atlas_w + q.x) * 4, (size_t)atlas_w * 4, q.key, (size_t)q.w * 4, (size_t)q.w * 4, q.h,
+            CK(r->err, cudaMemcpy2DAsync((char *)sl.atlas.p + ((size_t)q.y * atlas_w + q.x) * 4, (size_t)atlas_w * 4, q.key, (size_t)q.w * 4, (size_t)q.w * 4, q.h,
                                  cudaMemcpyHostToDevice, st));
-    CK(cudaGetLastError());
+    CK(r->err, cudaGetLastError());
     // the host vectors above are read by the asynchronous copies: they must outlive them
-    CK(cudaStreamSynchronize(st));
-    r->layout = L;
-    r->scene_words = total_words;
-    r->have_scene = true;
+    CK(r->err, cudaStreamSynchronize(st));
+    sl.layout = L;
+    sl.scene_words = total_words;
+    sl.have_scene = true;
     if (layout_out) memcpy(layout_out, &L, sizeof(vb_layout));
     return VB_OK;
 }
 
 
 // ---- multi-GPU exchange set-up (k_exchange.cu) ----------------------------------------------------------------------------
-// grow_arenas() is declared above; these entry points only manage the arena and the peer table.
+// These entry points only manage the arena and the peer table; an overflowing exchanged frame is grown by render_attempts.
 extern "C" int vb_exchange_configure(vb_renderer *r, uint32_t rank, uint32_t world, void **arena, size_t *arena_bytes) {
     if (!r || world < 1u || world > 8u || rank >= world) return VB_E_INVALID;
-    if (!r->have_scene) return VB_E_NO_SCENE;
-    CK(cudaSetDevice(r->device));
-    CK(cudaStreamSynchronize(r->stream));
+    const VbLayout &L = r->cur().layout;
+    if (!r->cur().have_scene) return VB_E_NO_SCENE;
+    CK(r->err, cudaSetDevice(r->device));
+    CK(r->err, cudaStreamSynchronize(r->stream));
     vb_renderer::Exchange &x = r->xc;
     x.enabled = false;
-    const uint32_t n_tags = (r->layout.path_data_base - r->layout.path_tag_base) * 4u;
+    const uint32_t n_tags = (L.path_data_base - L.path_tag_base) * 4u;
     // my outbox holds my share of the lines (+ the ones needed by two stripes): generous and fixed, so that the arena -- which
     // the peers have mapped -- never moves
     const uint64_t cap = (uint64_t)n_tags * 4u / world * 2u + 262144u;
     x.lines_cap = cap > 0x7fffffffull ? 0x7fffffffu : (uint32_t)cap;
-    x.n_paths = r->layout.n_paths;
+    x.n_paths = L.n_paths;
     x.half_bytes = vb_exchange_half_bytes(x.n_paths, x.lines_cap);
     const size_t bytes = 256 + 2 * x.half_bytes;
     int rc = ensure(r, x.arena, bytes);
     if (rc) return rc;
-    CK(cudaMemset(x.arena.p, 0, 256)); // flags and epoch start at 0
+    CK(r->err, cudaMemset(x.arena.p, 0, 256)); // flags and epoch start at 0
     x.rank = rank;
     x.world = world;
     memset(x.peer, 0, sizeof x.peer);

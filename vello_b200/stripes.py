@@ -52,7 +52,7 @@ def even_tile_bounds(world: int, height: int) -> List[int]:
 
 
 def rebalance(bounds: List[int], ms: List[float], damping: float = 0.5, tolerance: float = 0.06) -> List[int]:
-    """New boundaries from the device times of the last frame (same rule as group_rebalance in vb_api.cu): the cost of a
+    """New boundaries from the device times of the last frame (same rule as group_rebalance in vb_group.cu): the cost of a
     stripe is assumed to be spread evenly over its tile rows, the boundaries move (damped) to where the cumulative cost
     crosses k/n of the total; every stripe keeps at least one tile row. Unchanged when the times agree within `tolerance`."""
     n = len(ms)
